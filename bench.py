@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]           # our sm_100a path
     python bench.py --impl reference [...]                        # the LIVE reference's CPU path (oracle/_ref)
+    python bench.py --dump-outputs DIR [...]                      # + the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input: one
 fake-quant forward + one backward (incl. the in-kernel deterministic reduction) over a
@@ -77,7 +78,14 @@ def parse_args():
                          "step), and the fake-quant kernels walk dense NHWC storage directly, no copies")
     ap.add_argument("--no-eager-ref", action="store_true",
                     help="skip timing the reference's ATen chain on the GPU (second denominator)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed microbench steps, write what the last one returned (y, grad_x, grad_scale) "
+                         "as DIR/<name>.npy; an output above 2^22 elements is cut to a fixed seeded sample, "
+                         "saved flat")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the outputs of our timed path; it does not apply to --impl reference")
+    return a
 
 
 def peaks():
@@ -117,6 +125,23 @@ def make_inputs(a, device, log2n=None):
         scale = torch.exp2(torch.tensor([2.0 - a.bits], device=device))
         zp, lo, hi = b, b, b + 4.0 - scale
     return x, go, scale, zp, lo, hi
+
+
+DUMP_SAMPLE = 1 << 22      # elements kept of a larger output: 16 MB of fp32 per output
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as <out_dir>/<name>.npy in fp32.  One with more than DUMP_SAMPLE elements is
+    cut to the flat indices drawn by a CPU generator seeded 0, so that runs with the same arguments,
+    and different builds, write the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------
@@ -597,6 +622,10 @@ def run_ours(a):
     n_l = launches["n"]
     per_step = ms / a.steps
     gbs = world * (BYTES_FWD + BYTES_BWD) * n / (per_step * 1e-3) / 1e9
+    if a.dump_outputs and rank == 0:
+        # the last timed step's outputs (a replayed graph rewrites the tensors its capture kept)
+        y, gx, gs = keep["out"]
+        dump_outputs(a.dump_outputs, {"y": y, "grad_x": gx, "grad_scale": gs})
     if graph is not None:
         del graph
         ops.set_device_philox_state(None)

@@ -43,8 +43,8 @@ def _worker(rank, world, port, q):
     try:
         sys.path.insert(0, ROOT)
         import mhaq_b200
-        from oracle import ref_loader
-        ref = ref_loader.load_ops()
+        from oracle import ref_loader, ref_port
+        ref = ref_loader.load_ops() if ref_loader.available() else ref_port.load()
         orig_randint_like = torch.randint_like
 
         def run_case(shape, per_channel, tag):
@@ -171,9 +171,6 @@ def _worker(rank, world, port, q):
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
 def test_two_rank_nccl_aewgs_cuda_path_matches_the_live_reference():
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref not staged")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()

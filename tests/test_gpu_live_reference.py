@@ -1,5 +1,7 @@
 """GPU parity against the LIVE reference (oracle/_ref, the unmodified reference sources staged by
-oracle/make_ref.py) running ON THE SAME GPU, at the configurations the benchmarks measure.
+oracle/make_ref.py) running ON THE SAME GPU, at the configurations the benchmarks measure.  Where
+it is not staged, the same tests run against oracle/ref_port.py, the reference's API restated on
+the golden-pinned oracle.
 
 Bars (BASELINE.json north_star): fake-quant outputs / codes and STE / LSQ input gradients
 bit-exact; AEWGS input gradients 1e-5 relative (they depend on per-channel fp32 means);
@@ -16,7 +18,7 @@ import torch
 
 from oracle import checks as C
 from oracle import fq_oracle as O
-from oracle import ref_loader
+from oracle import ref_loader, ref_port
 
 pytestmark = pytest.mark.gpu
 
@@ -25,9 +27,8 @@ REL = 1e-5
 
 @pytest.fixture(scope="module")
 def ref():
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref not staged (run python oracle/make_ref.py where /root/reference exists)")
-    return ref_loader.load_ops()
+    # the live reference where oracle/_ref/ is staged, else its restatement on the oracle
+    return ref_loader.load_ops() if ref_loader.available() else ref_port.load()
 
 
 @pytest.fixture(scope="module")
