@@ -29,6 +29,10 @@
  *                              MinMaxObserver takes during calibration
  *                              (calib/minmaxobserver.py:28-37) — all from the forward's own pass
  *   mhaq_fq_noise_f32          torch.randint_like(input, 2).sub_(0.5)  (gdnsq.py:54)
+ *   mhaq_fq_pack_f32           the forward's integer codes stored at their real width (1, 2, 4, 8
+ *                              or 16 bits, "Packed codes" below): the low-bit artifact of QAT
+ *   mhaq_fq_unpack_f32         its inverse, code * s + zero_point, in every parameter mode
+ *   mhaq_fq_packed_row_bytes   the row stride of the packed format
  *   mhaq_fq_potential_loss_*   PotentialLoss.forward's constraint arithmetic and its autograd
  *                              (gdnsq_loss.py:32-86, 114-168), one launch each way
  *
@@ -325,6 +329,46 @@ int mhaq_fq_potential_loss_bwd_f32(const float *log_act_s, const float *log_act_
 int mhaq_fq_noise_f32(float *r, int64_t n_rows, int64_t n_inner,
                       uint64_t seed, uint64_t offset, const uint64_t *philox_dev,
                       void *stream);
+
+/* Packed codes.
+ *   Width b in {1, 2, 4, 8, 16}.  A learned width of 3, 5, 6 or 7 is stored in the next supported
+ *   width (the true width is the caller's to record).
+ *   The tensor is the usual [n_rows][n_inner] storage-order view, row r quantized with channel
+ *   r % n_ch; the stored value is the code rint(v) the forward computes (the same device
+ *   functions, so it is identical to mhaq_fq_fwd_f32's `codes` by construction).
+ *   Row r starts at byte r * row_stride, row_stride = round_up(ceil(n_inner * b / 8), 16), so every
+ *   row is 16-byte aligned (relative to the buffer).  For b <= 8, code j of a row occupies bits
+ *   [(j*b) mod 8, +b) of byte floor(j*b / 8), least-significant bit first; for b = 16 it is a
+ *   little-endian uint16 at byte 2j.  Padding bits and bytes are 0.
+ *   A code outside [0, 2^b - 1] (a NaN code included) is stored saturated (NaN as 0) and counted.
+ *   Only the generic operator can produce one: weight codes are >= 0 because the zero point is
+ *   the row minimum, and clamped activation codes are >= 0 as well.
+ *   Dequantization is y = code * s, then + zero_point: two roundings, as in the forward.  For every
+ *   in-range element y equals the forward's output bit for bit.  (A zero code is always +0 in the
+ *   forward too: v + (rint(v) - v) rounds to +0 for every v in (-0.5, 0], so a zero point of -0.0
+ *   gives +0 on both sides.)
+ *
+ * mhaq_fq_packed_row_bytes: row_stride for (n_inner, b), or -1 for a bad width / n_inner < 0. */
+int64_t mhaq_fq_packed_row_bytes(int64_t n_inner, int bits);
+
+/* Pack x's codes into `packed` (n_rows * mhaq_fq_packed_row_bytes(n_inner, bits) bytes, every byte
+ * written).  Parameters, strides, param_mode and the geometry are those of mhaq_fq_fwd_f32.
+ * n_out_of_range: NULL, or one device counter to which the number of saturated codes is ADDED
+ * (one integer atomic per CTA that saw any; the caller zeroes it).  No host synchronisation and
+ * no allocation: safe under CUDA-graph capture. */
+int mhaq_fq_pack_f32(const float *x, uint8_t *packed, int bits,
+                     const float *scale, const float *zp, const float *lo, const float *hi,
+                     int scale_stride, int zp_stride, int lo_stride, int hi_stride, int param_mode,
+                     int64_t n_rows, int64_t n_inner, int64_t n_ch,
+                     unsigned long long *n_out_of_range, void *stream);
+
+/* y = code * s + zp from packed codes, with s and zp as the forward forms them in `param_mode`
+ * (ACT_LOG: scale -> log_act_s, zp -> act_b; WEIGHT_LOG: scale -> log_wght_s[ch]; UNIT: y = code).
+ * Capture-safe like mhaq_fq_pack_f32. */
+int mhaq_fq_unpack_f32(const uint8_t *packed, int bits, float *y,
+                       const float *scale, const float *zp,
+                       int scale_stride, int zp_stride, int param_mode,
+                       int64_t n_rows, int64_t n_inner, int64_t n_ch, void *stream);
 
 #ifdef __cplusplus
 }

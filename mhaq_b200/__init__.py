@@ -6,8 +6,11 @@ ImportError, a CPU tensor is a RuntimeError.
 """
 from . import _lib  # noqa: F401  (fails loudly if the CUDA library is not built)
 from .ops import (  # noqa: F401
+    PackedCodes,
     fake_quant,
+    pack_codes,
     quantize_codes,
+    unpack_codes,
     quantize_eval,
     philox_noise,
     row_stats,
@@ -15,4 +18,4 @@ from .ops import (  # noqa: F401
 )
 
 __all__ = ["fake_quant", "quantize_codes", "quantize_eval", "philox_noise", "row_stats",
-           "set_device_philox_state"]
+           "set_device_philox_state", "PackedCodes", "pack_codes", "unpack_codes"]

@@ -70,6 +70,10 @@ _SIGNATURES = {
     "mhaq_fq_potential_loss_bwd_f32": (c_int, [_P, _P, c_int64, _P, _P, c_int64, _P, _P, c_float, c_float,
                                                c_float, _P, _P, _P, _P, _P, _P]),
     "mhaq_fq_noise_f32": (c_int, [_P, c_int64, c_int64, c_uint64, c_uint64, _P, _P]),
+    "mhaq_fq_packed_row_bytes": (c_int64, [c_int64, c_int]),
+    "mhaq_fq_pack_f32": (c_int, [_P, _P, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+                                 c_int64, c_int64, c_int64, _P, _P]),
+    "mhaq_fq_unpack_f32": (c_int, [_P, c_int, _P, _P, _P, c_int, c_int, c_int, c_int64, c_int64, c_int64, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

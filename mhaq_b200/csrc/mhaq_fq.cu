@@ -1516,6 +1516,7 @@ fq_rowstat_bwd_kernel(const float *__restrict__ gx, const float *__restrict__ x,
 
 #include "fq_wrow.cuh"
 #include "fq_loss.cuh"
+#include "fq_pack.cuh"
 
 // ===========================================================================
 // Host-side launch helpers
@@ -1757,6 +1758,31 @@ int wrow_multi_check(const mhaq_fq_wrow_bwd_desc *descs, int n_tensors, bool *ex
         else if ((d.r != nullptr) != *explicit_r) return MHAQ_FQ_EINVAL;   // all explicit or all in-kernel
     }
     return 0;
+}
+
+// ---- packed codes (fq_pack.cuh) ----
+inline bool pack_bits_ok(int bits) {
+    return bits == 1 || bits == 2 || bits == 4 || bits == 8 || bits == 16;
+}
+
+template <int BITS>
+void launch_pack(bool vec, bool clamp, int grid, cudaStream_t st, const float *x, uint8_t *packed,
+                 const QParams &prm, const Geom &g, int64_t row_stride, unsigned long long *n_oor) {
+    if (vec && clamp)
+        fq_pack_kernel<BITS, true, true><<<grid, kThreads, 0, st>>>(x, packed, prm, g, row_stride, n_oor);
+    else if (vec)
+        fq_pack_kernel<BITS, true, false><<<grid, kThreads, 0, st>>>(x, packed, prm, g, row_stride, n_oor);
+    else
+        fq_pack_kernel<BITS, false, true><<<grid, kThreads, 0, st>>>(x, packed, prm, g, row_stride, n_oor);
+}
+
+template <int BITS>
+void launch_unpack(bool vec, int grid, cudaStream_t st, const uint8_t *packed, float *y, const QParams &prm,
+                   const Geom &g, int64_t row_stride) {
+    if (vec)
+        fq_unpack_kernel<BITS, true><<<grid, kThreads, 0, st>>>(packed, y, prm, g, row_stride);
+    else
+        fq_unpack_kernel<BITS, false><<<grid, kThreads, 0, st>>>(packed, y, prm, g, row_stride);
 }
 
 }  // namespace
@@ -2203,6 +2229,67 @@ int mhaq_fq_potential_loss_bwd_f32(const float *log_act_s, const float *log_act_
     if (grid > 1024) grid = 1024;
     fq_potential_loss_bwd_kernel<<<grid, kLossThreads, 0, (cudaStream_t)stream>>>(
         a, saved, g_loss, g_log_act_s, g_log_act_q, g_log_wght_s, g_log_w_range, g_base_loss);
+    return last_error();
+}
+
+int64_t mhaq_fq_packed_row_bytes(int64_t n_inner, int bits) {
+    if (n_inner < 0 || !pack_bits_ok(bits)) return -1;
+    return packed_row_bytes(n_inner, bits);
+}
+
+int mhaq_fq_pack_f32(const float *x, uint8_t *packed, int bits, const float *scale, const float *zp,
+                     const float *lo, const float *hi, int scale_stride, int zp_stride, int lo_stride,
+                     int hi_stride, int param_mode, int64_t n_rows, int64_t n_inner, int64_t n_ch,
+                     unsigned long long *n_out_of_range, void *stream) {
+    int rc = check_common(x, scale, zp, n_rows, n_inner, n_ch);
+    if (rc) return rc;
+    if (!packed) return MHAQ_FQ_ENULL;
+    if (!pack_bits_ok(bits)) return MHAQ_FQ_EINVAL;
+    if ((rc = check_mode(param_mode, lo, n_ch)) != 0) return rc;
+    if (!stride_ok(scale_stride) || !stride_ok(zp_stride) || !stride_ok(lo_stride) ||
+        !stride_ok(hi_stride))
+        return MHAQ_FQ_EINVAL;
+    if (n_rows == 0 || n_inner == 0) return 0;
+    const Geom g = stream_geom(n_rows, n_inner, n_ch);
+    const QParams prm = {scale, zp, lo, hi, scale_stride, zp_stride, lo_stride, hi_stride, param_mode};
+    const bool vec = (n_inner % 4 == 0) && aligned16(x) && aligned16(packed);
+    const bool clamp = has_clamp(param_mode, lo, hi);
+    const int64_t rs = packed_row_bytes(n_inner, bits);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = grid_for(g.n_tasks);
+    switch (bits) {
+        case 1: launch_pack<1>(vec, clamp, grid, st, x, packed, prm, g, rs, n_out_of_range); break;
+        case 2: launch_pack<2>(vec, clamp, grid, st, x, packed, prm, g, rs, n_out_of_range); break;
+        case 4: launch_pack<4>(vec, clamp, grid, st, x, packed, prm, g, rs, n_out_of_range); break;
+        case 8: launch_pack<8>(vec, clamp, grid, st, x, packed, prm, g, rs, n_out_of_range); break;
+        default: launch_pack<16>(vec, clamp, grid, st, x, packed, prm, g, rs, n_out_of_range); break;
+    }
+    return last_error();
+}
+
+int mhaq_fq_unpack_f32(const uint8_t *packed, int bits, float *y, const float *scale, const float *zp,
+                       int scale_stride, int zp_stride, int param_mode, int64_t n_rows, int64_t n_inner,
+                       int64_t n_ch, void *stream) {
+    int rc = check_common(packed, scale, zp, n_rows, n_inner, n_ch);
+    if (rc) return rc;
+    if (!y) return MHAQ_FQ_ENULL;
+    if (!pack_bits_ok(bits) || !mode_ok(param_mode)) return MHAQ_FQ_EINVAL;
+    if (param_mode == PARAMS_ACT_LOG && n_ch != 1) return MHAQ_FQ_EINVAL;
+    if (!stride_ok(scale_stride) || !stride_ok(zp_stride)) return MHAQ_FQ_EINVAL;
+    if (n_rows == 0 || n_inner == 0) return 0;
+    const Geom g = stream_geom(n_rows, n_inner, n_ch);
+    const QParams prm = {scale, zp, nullptr, nullptr, scale_stride, zp_stride, 0, 0, param_mode};
+    const bool vec = (n_inner % 4 == 0) && aligned16(y) && aligned16(packed);
+    const int64_t rs = packed_row_bytes(n_inner, bits);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = grid_for(g.n_tasks);
+    switch (bits) {
+        case 1: launch_unpack<1>(vec, grid, st, packed, y, prm, g, rs); break;
+        case 2: launch_unpack<2>(vec, grid, st, packed, y, prm, g, rs); break;
+        case 4: launch_unpack<4>(vec, grid, st, packed, y, prm, g, rs); break;
+        case 8: launch_unpack<8>(vec, grid, st, packed, y, prm, g, rs); break;
+        default: launch_unpack<16>(vec, grid, st, packed, y, prm, g, rs); break;
+    }
     return last_error();
 }
 

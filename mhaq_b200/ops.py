@@ -9,6 +9,7 @@ forward and ONE in backward (plus a tiny finalize), through the C ABI in
 from __future__ import annotations
 
 import math
+from dataclasses import dataclass
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -1062,3 +1063,113 @@ def potential_loss(base_loss, las, laq, lws, lwq, loss_sum, cnt, wt, at, eps, t,
         _require_cuda(v)
     return _PotentialLossFn.apply(base_loss.reshape(()), las, laq, lws, lwq, loss_sum, cnt, wt, at, eps, t,
                                   lossless, training)
+
+
+# ---------------------------------------------------------------------------------------------
+# Packed integer codes (include/mhaq_fq.h: "Packed codes", mhaq_fq_pack_f32 / mhaq_fq_unpack_f32):
+# the codes the forward computes, stored at 1, 2, 4, 8 or 16 bits with the scale and zero point
+# that turn them back into the fake-quantized tensor.
+# ---------------------------------------------------------------------------------------------
+PACK_BITS = (1, 2, 4, 8, 16)
+
+
+@dataclass
+class PackedCodes:
+    """Codes of one tensor in the packed format of include/mhaq_fq.h.
+
+    ``data`` is uint8 ``[n_rows, row_stride]`` over the ``[n_rows][n_inner]`` storage-order view
+    (row r quantized with channel r % n_ch); ``shape`` / ``stride`` are those of the packed tensor,
+    so ``unpack_codes`` returns the same layout.  ``scale`` / ``zero_point`` are the flattened
+    operands the codes were made with, interpreted by parameter mode ``mode`` (log-domain for the
+    layer forms).  ``n_out_of_range`` is a device counter of the codes that had to be saturated."""
+    data: torch.Tensor
+    bits: int
+    shape: Tuple[int, ...]
+    stride: Tuple[int, ...]
+    n_rows: int
+    n_inner: int
+    n_ch: int
+    scale: torch.Tensor
+    zero_point: torch.Tensor
+    n_out_of_range: torch.Tensor
+    mode: int = PARAMS_LINEAR
+
+
+def packed_row_bytes(n_inner: int, bits: int) -> int:
+    """Bytes per packed row: round_up(ceil(n_inner * bits / 8), 16)."""
+    n = int(lib.mhaq_fq_packed_row_bytes(n_inner, bits))
+    if n < 0:
+        raise ValueError(f"packed codes: bits must be one of {PACK_BITS}, got {bits}")
+    return n
+
+
+def _smallest_bits(x, L: _Launch) -> int:
+    """Width for the codes' range, from the statistics-only forward (one host read)."""
+    _, _, mm = _forward_impl(x, L, want_y=False, want_codes=False, want_minmax=True)
+    cmin, cmax, bad = mm[:3].tolist()
+    if bad != 0 or cmin < 0:
+        raise ValueError(f"packed codes: codes span [{cmin}, {cmax}]; no unsigned width holds them")
+    for b in PACK_BITS:
+        if cmax <= (1 << b) - 1:
+            return b
+    raise ValueError(f"packed codes: the largest code {cmax:.0f} needs more than 16 bits")
+
+
+def _pack(x, L: _Launch, bits, check_range: bool) -> PackedCodes:
+    geo = L.geo
+    if bits is None:
+        bits = _smallest_bits(x, L) if x.numel() else PACK_BITS[0]
+    row = packed_row_bytes(geo.n_inner, bits)
+    data = torch.empty(geo.n_rows, row, dtype=torch.uint8, device=x.device)
+    n_bad = torch.zeros(1, dtype=torch.int64, device=x.device)      # unsigned long long counter
+    if x.numel():
+        check(lib.mhaq_fq_pack_f32(_ptr(x), _ptr(data), bits, *L.params(), geo.n_rows, geo.n_inner,
+                                   geo.n_ch, _ptr(n_bad), _stream()), "mhaq_fq_pack_f32")
+    p = PackedCodes(data, bits, tuple(x.shape), tuple(x.stride()), geo.n_rows, geo.n_inner, geo.n_ch,
+                    L.scale, L.zp, n_bad, L.mode)
+    if check_range:
+        n = int(n_bad.item())
+        if n:
+            raise ValueError(f"packed codes: {n} code(s) outside [0, {(1 << bits) - 1}] (NaN included)")
+    return p
+
+
+def pack_codes(x, scale, zero_point, min_val=None, max_val=None, bits=None, check=True) -> PackedCodes:
+    """The codes ``quantize_codes`` returns, packed at ``bits`` (1, 2, 4, 8 or 16) per code.
+
+    Parameters are interpreted exactly as ``fake_quant`` interprets them.  ``bits=None`` picks the
+    smallest width that holds [min code, max code] (one statistics pass and one host read; raises
+    if no width fits).  ``check=True`` reads the out-of-range counter once and raises ValueError if
+    any code had to be saturated; ``check=False`` synchronises nothing (CUDA-graph capture, which
+    also needs an explicit ``bits``)."""
+    x = x.detach()
+    L = _Launch(x, scale, zero_point, min_val, max_val)
+    return _pack(_dense(x, L.geo.axis), L, bits, check)
+
+
+def pack_act_codes(x, log_act_s, log_act_q, act_b, bits=None, check=True) -> PackedCodes:
+    """``pack_codes`` with NoisyAct's parameters (s = 2^log_act_s, zero point = min_val = act_b,
+    max_val = (act_b + 2^log_act_q) - s, formed in the kernel as the layer's forward forms them)."""
+    x = x.detach()
+    L = _Launch.act_log(x, log_act_s, log_act_q, act_b)
+    return _pack(_dense(x, None), L, bits, check)
+
+
+def pack_weight_codes(w, log_wght_s, row_min, bits=None, check=True) -> PackedCodes:
+    """``pack_codes`` for a per-channel (dim 0) weight from its log scale and row minimum, as the
+    layers' fused weight path forms them (s = 2^log_wght_s[row], zero point = row_min[row])."""
+    w = _dense(w.detach(), 0)
+    L = _Launch.weight_log(w, log_wght_s, row_min)
+    return _pack(w, L, bits, check)
+
+
+def unpack_codes(p: PackedCodes) -> torch.Tensor:
+    """code * s + zero_point for every element of ``p``, fp32 with ``p``'s shape and strides: for
+    every code that was in range, bit for bit the output of the forward the codes came from."""
+    y = torch.empty_strided(p.shape, p.stride, dtype=torch.float32, device=p.data.device)
+    if y.numel():
+        ss = 0 if p.scale.numel() == 1 else 1
+        zs = 0 if p.zero_point.numel() == 1 else 1
+        check(lib.mhaq_fq_unpack_f32(_ptr(p.data), p.bits, _ptr(y), _ptr(p.scale), _ptr(p.zero_point), ss, zs,
+                                     p.mode, p.n_rows, p.n_inner, p.n_ch, _stream()), "mhaq_fq_unpack_f32")
+    return y
