@@ -33,6 +33,11 @@
  *                              or 16 bits, "Packed codes" below): the low-bit artifact of QAT
  *   mhaq_fq_unpack_f32         its inverse, code * s + zero_point, in every parameter mode
  *   mhaq_fq_packed_row_bytes   the row stride of the packed format
+ *   mhaq_fq_act_codes_f32      the activation codes of an eval-mode NoisyAct as uint8, channels padded
+ *                              to 16: the input of the integer layers ("Integer layers" below)
+ *   mhaq_fq_iconv_u8           a quantized convolution / linear layer on integer codes: int8
+ *                              tensor-core implicit GEMM (tcgen05.mma kind::i8), fp32 output
+ *   mhaq_fq_iconv_weight_bytes the size and tiling of the weight operand mhaq_fq_iconv_u8 reads
  *   mhaq_fq_potential_loss_*   PotentialLoss.forward's constraint arithmetic and its autograd
  *                              (gdnsq_loss.py:32-86, 114-168), one launch each way
  *
@@ -369,6 +374,50 @@ int mhaq_fq_unpack_f32(const uint8_t *packed, int bits, float *y,
                        const float *scale, const float *zp,
                        int scale_stride, int zp_stride, int param_mode,
                        int64_t n_rows, int64_t n_inner, int64_t n_ch, void *stream);
+
+/* Integer layers.
+ *   A quantized layer y = conv(a, w) + bias (a Linear is the case H = W = kh = kw = 1) with
+ *   a = ca * sa + zpa (activation code ca in [0, act_max_code]) and w_nk = cw_nk * sw_n + zpw_n
+ *   (weight code cw in [0, weight_max_code]) is evaluated as
+ *     y[m][n] = alpha[n] * S[m][n] + beta[n] * SA[m] + ctab[p(m)][n]
+ *   with S = sum over the valid taps k of ca_k * cw_nk and SA = sum of ca_k (both int32, exact),
+ *   alpha = sa * sw, beta = sa * zpw and ctab[p][n] = zpa * (sw_n * sum_{k in p} cw_nk + zpw_n * |p|)
+ *   + bias_n for the pixel's tap-validity pattern p(m) = h_class[ho] * n_w_classes + w_class[wo]
+ *   (DESIGN.md §3).  A padding tap is the value 0, so it adds nothing to any of the three terms.
+ *   The epilogue evaluates the sum in fp64 and rounds once to fp32.
+ *
+ * mhaq_fq_act_codes_f32: codes[pixel][c] = the forward's code of x[pixel][c] (clamped to
+ *   [zero_point, max_val], per-tensor LINEAR parameters, one float each), saturated to [0, 255]
+ *   (NaN -> 0) and counted into *n_out_of_range (NULL = not counted) like mhaq_fq_pack_f32;
+ *   channels [n_channels, cp) are 0.  x is [n_pixels][n_channels] (channels_last NCHW storage or a
+ *   [B, in] matrix); codes is [n_pixels][cp], cp % 16 == 0, 16-byte aligned.
+ *
+ * mhaq_fq_iconv_weight_bytes: bytes of the weight operand for n_out output channels and K =
+ *   k_bytes = kh * kw * cp; -1 for a bad size.  The operand holds n_tiles tiles of tile_n rows
+ *   (tile_n % 16 == 0, <= 256): tile t has output channels [t * tile_out, min(n_out, (t+1) *
+ *   tile_out)), tile_out <= 255 and no tile empty, then one row of ones (it yields SA), then zero
+ *   rows.  A row is K bytes in
+ *   (kh, kw, cp) order, zero-padded to k_stages * 128.  Storage: [tile][stage][tile_n * 128], the
+ *   byte of row r and K position 16 * c + j (0 <= c < 8, 0 <= j < 16) of a stage at
+ *   (r / 8) * 1024 + c * 128 + (r % 8) * 16 + j.  Any output pointer may be NULL.
+ *
+ * mhaq_fq_iconv_u8: codes from mhaq_fq_act_codes_f32 ([batch][height][width][cp], 16-byte
+ *   aligned), the weight operand above (16-byte aligned), alpha / beta [n_out], ctab
+ *   [n_h_classes * n_w_classes][n_out], h_class [ho], w_class [wo] (int32); y is fp32
+ *   [batch * ho * wo][n_out] (a channels_last [batch, n_out, ho, wo] or a [batch, n_out] tensor).
+ *   Errors (before any CUDA call): cp % 16 != 0, bad sizes, a code bound outside [1, 255], and
+ *   kh * kw * cp * act_max_code * weight_max_code >= 2^31 (the int32 accumulator could overflow).
+ *   Capture-safe: no host synchronisation, allocation or atomic. */
+int64_t mhaq_fq_iconv_weight_bytes(int64_t n_out, int64_t k_bytes, int *n_tiles, int *tile_n, int *tile_out,
+                                   int64_t *k_stages);
+int mhaq_fq_act_codes_f32(const float *x, uint8_t *codes, const float *scale, const float *zero_point,
+                          const float *max_val, int64_t n_pixels, int64_t n_channels, int64_t cp,
+                          unsigned long long *n_out_of_range, void *stream);
+int mhaq_fq_iconv_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                     const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                     float *y, int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
+                     int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                     int act_max_code, int weight_max_code, void *stream);
 
 #ifdef __cplusplus
 }

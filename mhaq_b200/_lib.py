@@ -74,6 +74,10 @@ _SIGNATURES = {
     "mhaq_fq_pack_f32": (c_int, [_P, _P, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
                                  c_int64, c_int64, c_int64, _P, _P]),
     "mhaq_fq_unpack_f32": (c_int, [_P, c_int, _P, _P, _P, c_int, c_int, c_int, c_int64, c_int64, c_int64, _P]),
+    "mhaq_fq_iconv_weight_bytes": (c_int64, [c_int64, c_int64, _P, _P, _P, _P]),
+    "mhaq_fq_act_codes_f32": (c_int, [_P, _P, _P, _P, _P, c_int64, c_int64, c_int64, _P, _P]),
+    "mhaq_fq_iconv_u8": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int64, c_int64, c_int64, c_int64,
+                                 c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

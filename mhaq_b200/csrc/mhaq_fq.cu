@@ -1517,6 +1517,7 @@ fq_rowstat_bwd_kernel(const float *__restrict__ gx, const float *__restrict__ x,
 #include "fq_wrow.cuh"
 #include "fq_loss.cuh"
 #include "fq_pack.cuh"
+#include "fq_igemm.cuh"
 
 // ===========================================================================
 // Host-side launch helpers
@@ -1783,6 +1784,21 @@ void launch_unpack(bool vec, int grid, cudaStream_t st, const uint8_t *packed, f
         fq_unpack_kernel<BITS, true><<<grid, kThreads, 0, st>>>(packed, y, prm, g, row_stride);
     else
         fq_unpack_kernel<BITS, false><<<grid, kThreads, 0, st>>>(packed, y, prm, g, row_stride);
+}
+
+// ---- integer layers (fq_igemm.cuh) ----
+// The iconv kernel needs more than 48 KiB of dynamic shared memory: opt in once per device.
+inline int iconv_smem_opt_in() {
+    static bool done[64] = {};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return (int)e;
+    if (dev < 64 && done[dev]) return 0;
+    e = cudaFuncSetAttribute(fq_iconv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)iconv_smem_bytes(kIcMaxTileN));
+    if (e != cudaSuccess) return (int)e;
+    if (dev < 64) done[dev] = true;
+    return 0;
 }
 
 }  // namespace
@@ -2301,6 +2317,76 @@ int mhaq_fq_noise_f32(float *r, int64_t n_rows, int64_t n_inner, uint64_t seed, 
     const Geom g = stream_geom(n_rows, n_inner, 1);
     fq_noise_kernel<<<grid_for(g.n_tasks), kThreads, 0, (cudaStream_t)stream>>>(r, g, seed, offset,
                                                                                philox_dev);
+    return last_error();
+}
+
+int64_t mhaq_fq_iconv_weight_bytes(int64_t n_out, int64_t k_bytes, int *n_tiles, int *tile_n, int *tile_out,
+                                   int64_t *k_stages) {
+    if (n_out < 1 || k_bytes < 16 || k_bytes % 16 != 0) return -1;
+    const IcLayout l = iconv_layout(n_out, k_bytes);
+    if (n_tiles) *n_tiles = l.n_tiles;
+    if (tile_n) *tile_n = l.tile_n;
+    if (tile_out) *tile_out = l.tile_out;
+    if (k_stages) *k_stages = l.k_stages;
+    return (int64_t)l.n_tiles * l.k_stages * l.tile_n * kIcStageK;
+}
+
+int mhaq_fq_act_codes_f32(const float *x, uint8_t *codes, const float *scale, const float *zero_point,
+                          const float *max_val, int64_t n_pixels, int64_t n_channels, int64_t cp,
+                          unsigned long long *n_out_of_range, void *stream) {
+    if (!x || !codes || !scale || !zero_point || !max_val) return MHAQ_FQ_ENULL;
+    if (n_pixels < 0 || n_channels < 1 || cp < n_channels || cp % 16 != 0 || !aligned16(codes))
+        return MHAQ_FQ_EINVAL;
+    if (n_pixels == 0) return 0;
+    const QParams prm = {scale, zero_point, zero_point, max_val, 0, 0, 0, 0, PARAMS_LINEAR};
+    const bool vec = n_channels % 4 == 0 && aligned16(x);
+    const int64_t groups = n_pixels * (cp / 4);
+    const int64_t blocks = (groups + kThreads - 1) / kThreads;
+    const int grid = (int)(blocks < 148 * 64 ? blocks : 148 * 64);
+    fq_act_codes_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(x, codes, prm, n_pixels, n_channels, cp, vec,
+                                                                      n_out_of_range);
+    return last_error();
+}
+
+int mhaq_fq_iconv_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                     const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                     float *y, int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
+                     int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                     int act_max_code, int weight_max_code, void *stream) {
+    if (!codes || !weights || !alpha || !beta || !ctab || !h_class || !w_class || !y) return MHAQ_FQ_ENULL;
+    if (batch < 1 || height < 1 || width < 1 || cp < 16 || cp % 16 != 0 || n_out < 1 || n_w_classes < 1)
+        return MHAQ_FQ_EINVAL;
+    if (kernel_h < 1 || kernel_w < 1 || stride_h < 1 || stride_w < 1 || pad_h < 0 || pad_w < 0)
+        return MHAQ_FQ_EINVAL;
+    if (act_max_code < 1 || act_max_code > 255 || weight_max_code < 1 || weight_max_code > 255)
+        return MHAQ_FQ_EINVAL;
+    if (!aligned16(codes) || !aligned16(weights)) return MHAQ_FQ_EINVAL;
+    const int64_t ho = (height + 2 * pad_h - kernel_h) / stride_h + 1;
+    const int64_t wo = (width + 2 * pad_w - kernel_w) / stride_w + 1;
+    if (height + 2 * pad_h < kernel_h || width + 2 * pad_w < kernel_w) return MHAQ_FQ_EINVAL;
+    const int64_t k_bytes = (int64_t)kernel_h * kernel_w * cp;
+    // the int32 accumulator holds sum_k ca_k * cw_nk <= K * act_max_code * weight_max_code
+    if (k_bytes > (int64_t)1 << 31 || k_bytes * act_max_code * weight_max_code >= ((int64_t)1 << 31))
+        return MHAQ_FQ_EINVAL;
+    const IcLayout l = iconv_layout(n_out, k_bytes);
+    if (l.tile_n > kIcMaxTileN) return MHAQ_FQ_EINVAL;
+    const int64_t m = batch * ho * wo;
+    const int64_t m_tiles = (m + kIcTileM - 1) / kIcTileM;
+    if (m_tiles > 0x7fffffffLL) return MHAQ_FQ_EINVAL;
+    int rc = iconv_smem_opt_in();
+    if (rc) return rc;
+    IConvArgs a;
+    a.a = codes; a.b = weights; a.alpha = alpha; a.beta = beta; a.ctab = ctab;
+    a.hcls = h_class; a.wcls = w_class; a.y = y;
+    a.m = m; a.h = height; a.w = width; a.cp = cp; a.n_out = n_out; a.ho = ho; a.wo = wo;
+    a.k_chunks = k_bytes / 16; a.k_stages = l.k_stages;
+    a.kh = kernel_h; a.kw = kernel_w; a.sh = stride_h; a.sw = stride_w; a.ph = pad_h; a.pw = pad_w;
+    a.n_wcls = n_w_classes; a.tile_n = l.tile_n; a.tile_out = l.tile_out;
+    a.tmem_cols = 32;
+    while (a.tmem_cols < l.tile_n) a.tmem_cols <<= 1;
+    a.vec_out = aligned16(y) && n_out % 4 == 0;
+    const dim3 grid((unsigned)m_tiles, (unsigned)l.n_tiles);
+    fq_iconv_kernel<<<grid, kIcThreads, iconv_smem_bytes(l.tile_n), (cudaStream_t)stream>>>(a);
     return last_error();
 }
 

@@ -8,6 +8,7 @@ forward and ONE in backward (plus a tiny finalize), through the C ABI in
 """
 from __future__ import annotations
 
+import ctypes
 import math
 from dataclasses import dataclass
 from typing import Optional, Sequence, Tuple
@@ -16,6 +17,8 @@ import torch
 import torch.distributed as dist
 
 from ._lib import lib, check
+
+_check_rc = check   # for functions whose `check` argument shadows it
 
 METHOD_IDS = {"STE": 0, "EWGS": 1, "AEWGS": 2, "LSQ": 3}
 
@@ -1173,3 +1176,208 @@ def unpack_codes(p: PackedCodes) -> torch.Tensor:
         check(lib.mhaq_fq_unpack_f32(_ptr(p.data), p.bits, _ptr(y), _ptr(p.scale), _ptr(p.zero_point), ss, zs,
                                      p.mode, p.n_rows, p.n_inner, p.n_ch, _stream()), "mhaq_fq_unpack_f32")
     return y
+
+
+# ---------------------------------------------------------------------------------------------
+# Integer layers (include/mhaq_fq.h "Integer layers", DESIGN §3): a quantized convolution or
+# linear layer evaluated on the activation and weight codes with the int8 tensor cores,
+#   y[m][n] = alpha[n] * S[m][n] + beta[n] * SA[m] + ctab[p(m)][n].
+# ---------------------------------------------------------------------------------------------
+def code_channels(c: int) -> int:
+    """Channels of an activation-code row: C rounded up to 16 (the MMA K granularity is 32 bytes
+    per instruction and every 16-byte chunk of K must lie within one tap)."""
+    return (c + 15) // 16 * 16
+
+
+def act_codes(x, scale, zero_point, max_val, check=False):
+    """uint8 codes of an eval-mode ``NoisyAct`` with operands (scale, zero_point = min_val,
+    max_val), each one element: the forward's own codes, saturated to [0, 255] (NaN -> 0).
+
+    ``x`` is a 4-D tensor (taken channels_last; other layouts are copied) or a ``[B, in]``
+    matrix.  Returns ``(codes, n_out_of_range)``: codes ``[B, H, W, Cp]`` resp. ``[B, Cp]``,
+    Cp = ``code_channels(C)``, padding channels 0, and a device counter of saturated codes.
+    ``check=True`` reads the counter (one host synchronisation) and raises ValueError if it is
+    not zero."""
+    x = x.detach()
+    _require_cuda(x)
+    if x.dim() == 4:
+        x = x.contiguous(memory_format=torch.channels_last)
+        b, c, h, w = x.shape
+        lead = (b, h, w)
+    elif x.dim() == 2:
+        x = x.contiguous()
+        (b, c), lead = x.shape, (x.shape[0],)
+    else:
+        raise ValueError(f"act_codes: expected a 4-D or 2-D input, got shape {tuple(x.shape)}")
+    cp = code_channels(c)
+    codes = torch.empty(*lead, cp, dtype=torch.uint8, device=x.device)
+    n_bad = torch.zeros(1, dtype=torch.int64, device=x.device)      # unsigned long long counter
+    prm = [_prep_param(p, x, n)[0] for p, n in ((scale, "scale"), (zero_point, "zp"), (max_val, "hi_param"))]
+    if any(p.numel() != 1 for p in prm):
+        raise ValueError("act_codes: scale, zero_point and max_val must have one element each")
+    n_pix = x.numel() // c if c else 0
+    _check_rc(lib.mhaq_fq_act_codes_f32(_ptr(x), _ptr(codes), *(_ptr(p) for p in prm), n_pix, c, cp,
+                                        _ptr(n_bad), _stream()), "mhaq_fq_act_codes_f32")
+    if check:
+        n = int(n_bad.item())
+        if n:
+            raise ValueError(f"act_codes: {n} code(s) outside [0, 255] (NaN included)")
+    return codes, n_bad
+
+
+def iconv_layout(n_out: int, k_bytes: int):
+    """(bytes, n_tiles, tile_n, tile_out, k_stages) of the weight operand (mhaq_fq_iconv_weight_bytes)."""
+    nt, tn, to, ks = ctypes.c_int(), ctypes.c_int(), ctypes.c_int(), ctypes.c_int64()
+    n = int(lib.mhaq_fq_iconv_weight_bytes(n_out, k_bytes, ctypes.byref(nt), ctypes.byref(tn),
+                                           ctypes.byref(to), ctypes.byref(ks)))
+    if n < 0:
+        raise ValueError(f"iconv_layout: bad sizes n_out={n_out}, k_bytes={k_bytes}")
+    return n, nt.value, tn.value, to.value, ks.value
+
+
+def iconv_weight_operand(cw: torch.Tensor) -> torch.Tensor:
+    """The weight operand of mhaq_fq_iconv_u8 from integer weight codes ``cw [N, C, kh, kw]``:
+    flat uint8, rows (kh, kw, Cp) with zero padding channels, an all-ones row after each tile's
+    output channels, every (tile, stage) block in the kernel's shared-memory order."""
+    n, c, kh, kw = cw.shape
+    cp = code_channels(c)
+    k = kh * kw * cp
+    nbytes, nt, tn, to, ks = iconv_layout(n, k)
+    w = torch.zeros(n, kh, kw, cp, dtype=torch.uint8, device=cw.device)
+    w[..., :c] = cw.permute(0, 2, 3, 1).to(torch.uint8)
+    w = w.reshape(n, k)
+    rows = torch.zeros(nt, tn, ks * 128, dtype=torch.uint8, device=cw.device)
+    for t in range(nt):
+        lo, hi = t * to, min(n, (t + 1) * to)
+        rows[t, :hi - lo, :k] = w[lo:hi]
+        rows[t, to, :] = 1
+    # [tile][row group][row % 8][stage][chunk][byte] -> [tile][stage][row group][chunk][row % 8][byte]
+    out = rows.view(nt, tn // 8, 8, ks, 8, 16).permute(0, 3, 1, 4, 2, 5).reshape(-1)
+    assert out.numel() == nbytes
+    return out
+
+
+def tap_classes(size: int, k: int, stride: int, pad: int):
+    """Tap-validity classes along one axis: (class of each output position (int32 [out]),
+    valid taps of each class (bool [n_classes, k]))."""
+    out = (size + 2 * pad - k) // stride + 1
+    pos = torch.arange(out)[:, None] * stride - pad + torch.arange(k)[None, :]
+    valid = ((pos >= 0) & (pos < size)).to(torch.uint8)
+    uniq, inv = torch.unique(valid, dim=0, return_inverse=True)
+    return inv.to(torch.int32), uniq.bool()
+
+
+@dataclass
+class IntLayerOperands:
+    """Device operands of one integer layer (``int_layer_operands``).  ``weight``, ``alpha`` and
+    ``beta`` are fixed; the pattern tables depend on the input size and are built on first use
+    of each (H, W, stride, padding) and cached."""
+    weight: torch.Tensor          # uint8 operand (iconv_weight_operand)
+    alpha: torch.Tensor           # fp32 [N]: sa * sw
+    beta: torch.Tensor            # fp32 [N]: sa * zpw
+    n_out: int
+    cin: int
+    kh: int
+    kw: int
+    a_top: int                    # largest activation code
+    w_top: int                    # largest weight code
+    tap_sums: torch.Tensor        # fp64 [N, kh, kw]: sum over the channels of cw
+    sw: torch.Tensor              # fp64 [N]
+    zpw: torch.Tensor             # fp64 [N]
+    zpa: float
+    bias: Optional[torch.Tensor]  # fp64 [N] or None
+    tables: dict
+
+    @property
+    def cp(self) -> int:
+        return code_channels(self.cin)
+
+    def constant_table(self, hvalid: torch.Tensor, wvalid: torch.Tensor) -> torch.Tensor:
+        """fp64 ctab [n_h_classes * n_w_classes][N]: zpa * (sw * sum_{k in p} cw + zpw * |p|) + bias."""
+        mask = (hvalid[:, None, :, None] & wvalid[None, :, None, :]).to(torch.float64)
+        mask = mask.to(self.tap_sums.device)
+        wsum = torch.einsum("hwab,nab->hwn", mask, self.tap_sums)
+        cnt = mask.sum((2, 3))[..., None] * self.cin
+        c = self.zpa * (self.sw * wsum + self.zpw * cnt)
+        if self.bias is not None:
+            c = c + self.bias
+        return c.reshape(-1, self.n_out)
+
+    def pattern_tables(self, h: int, w: int, stride, padding):
+        """(h_class int32 [Ho], w_class int32 [Wo], n_w_classes, ctab fp32) on the operands' device."""
+        key = (h, w, tuple(stride), tuple(padding))
+        t = self.tables.get(key)
+        if t is None:
+            hc, hv = tap_classes(h, self.kh, stride[0], padding[0])
+            wc, wv = tap_classes(w, self.kw, stride[1], padding[1])
+            dev = self.weight.device
+            t = self.tables[key] = (hc.to(dev), wc.to(dev), wv.shape[0],
+                                    self.constant_table(hv, wv).to(device=dev, dtype=torch.float32).contiguous())
+        return t
+
+
+def int32_bound_ok(k_bytes: int, a_top: int, w_top: int) -> bool:
+    """The int32 accumulator holds every sum: K * a_top * w_top < 2^31 (K counts padding channels)."""
+    return k_bytes * a_top * w_top < (1 << 31)
+
+
+def int_layer_operands(cw, sw, zpw, sa, zpa, bias, a_top: int, w_top: int) -> IntLayerOperands:
+    """Operands of an integer layer on ``cw``'s device from the weight codes ``cw [N, C, kh, kw]``
+    (integers in [0, w_top]), the weight scale / zero point (``[N]`` or one element), the
+    activation scale / zero point (floats) and the layer's bias (``[N]`` or None).  alpha and beta
+    are formed in fp64 and rounded once to fp32."""
+    n, c, kh, kw = cw.shape
+    if not (1 <= a_top <= 255 and 1 <= w_top <= 255):
+        raise ValueError(f"integer layer: code bounds must lie in [1, 255], got {a_top} and {w_top}")
+    if not int32_bound_ok(kh * kw * code_channels(c), a_top, w_top):
+        raise ValueError("integer layer: K * (n_levels - 1) * (2^bits - 1) >= 2^31 would overflow the "
+                         "int32 accumulator")
+    dev = cw.device
+    f64 = dict(dtype=torch.float64, device=dev)
+    sw = torch.as_tensor(sw).to(**f64).reshape(-1).expand(n).contiguous()
+    zpw = torch.as_tensor(zpw).to(**f64).reshape(-1).expand(n).contiguous()
+    sa, zpa = float(sa), float(zpa)
+    return IntLayerOperands(
+        weight=iconv_weight_operand(cw), alpha=(sa * sw).float(), beta=(sa * zpw).float(),
+        n_out=n, cin=c, kh=kh, kw=kw, a_top=a_top, w_top=w_top,
+        tap_sums=cw.to(**f64).sum(1), sw=sw, zpw=zpw, zpa=zpa,
+        bias=None if bias is None else torch.as_tensor(bias).to(**f64).reshape(n),
+        tables={})
+
+
+def _iconv(codes, L: IntLayerOperands, y, b, h, w, stride, padding):
+    hc, wc, nwc, ctab = L.pattern_tables(h, w, stride, padding)
+    if codes.shape[-1] != L.cp or codes.dtype != torch.uint8 or not codes.is_contiguous():
+        raise ValueError(f"integer layer: expected contiguous uint8 codes with {L.cp} channels, "
+                         f"got {codes.dtype} {tuple(codes.shape)}")
+    if y.numel():
+        _check_rc(lib.mhaq_fq_iconv_u8(_ptr(codes), _ptr(L.weight), _ptr(L.alpha), _ptr(L.beta), _ptr(ctab),
+                                       _ptr(hc), _ptr(wc), nwc, _ptr(y), b, h, w, L.cp, L.n_out, L.kh, L.kw,
+                                       stride[0], stride[1], padding[0], padding[1], L.a_top, L.w_top,
+                                       _stream()), "mhaq_fq_iconv_u8")
+    return y
+
+
+def _pair(v):
+    return (int(v), int(v)) if isinstance(v, int) else (int(v[0]), int(v[1]))
+
+
+def int_conv2d(codes, L: IntLayerOperands, stride=1, padding=0) -> torch.Tensor:
+    """fp32 convolution of activation codes ``[B, H, W, Cp]`` (``act_codes``) with the layer's
+    operands: a channels_last ``[B, N, Ho, Wo]`` tensor."""
+    b, h, w, _ = codes.shape
+    stride, padding = _pair(stride), _pair(padding)
+    ho = (h + 2 * padding[0] - L.kh) // stride[0] + 1
+    wo = (w + 2 * padding[1] - L.kw) // stride[1] + 1
+    y = torch.empty((b, L.n_out, ho, wo), dtype=torch.float32, device=codes.device,
+                    memory_format=torch.channels_last)
+    return _iconv(codes, L, y, b, h, w, stride, padding)
+
+
+def int_linear(codes, L: IntLayerOperands) -> torch.Tensor:
+    """fp32 ``[B, N]`` linear layer on activation codes ``[B, Cp]`` (``act_codes``)."""
+    if L.kh != 1 or L.kw != 1:
+        raise ValueError("int_linear: the operands are those of a convolution")
+    b = codes.shape[0]
+    y = torch.empty((b, L.n_out), dtype=torch.float32, device=codes.device)
+    return _iconv(codes, L, y, b, 1, 1, (1, 1), (0, 0))

@@ -179,3 +179,6 @@ def load_quantized(model, blob) -> None:
             _load_act(name, m, e)
         else:
             _load_weight(name, m, e)
+
+
+from .inference import build_integer_model  # noqa: E402,F401  (runs an export on its integer codes)
