@@ -38,6 +38,9 @@
  *   mhaq_fq_iconv_u8           a quantized convolution / linear layer on integer codes: int8
  *                              tensor-core implicit GEMM (tcgen05.mma kind::i8), fp32 output
  *   mhaq_fq_iconv_weight_bytes the size and tiling of the weight operand mhaq_fq_iconv_u8 reads
+ *   mhaq_fq_iconv_fused_u8     mhaq_fq_iconv_u8 with an eval BatchNorm folded into its operands and
+ *                              the residual add, ReLU / LeakyReLU and the next layer's codes in its
+ *                              epilogue
  *   mhaq_fq_potential_loss_*   PotentialLoss.forward's constraint arithmetic and its autograd
  *                              (gdnsq_loss.py:32-86, 114-168), one launch each way
  *
@@ -418,6 +421,45 @@ int mhaq_fq_iconv_u8(const uint8_t *codes, const uint8_t *weights, const float *
                      float *y, int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
                      int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                      int act_max_code, int weight_max_code, void *stream);
+
+/* Fused epilogue of an integer convolution.
+ *   t = RN32(alpha * S + beta * SA + C) as in mhaq_fq_iconv_u8 (an eval BatchNorm k * y + shift is
+ *   folded into alpha, beta and C by the caller: DESIGN.md §3 "Fused epilogue"), then
+ *     residual   (optional) t = t + residual[m][n], one fp32 rounding; residual is fp32 [m][n_out],
+ *                the same storage-order view as y;
+ *     activation MHAQ_FQ_ACT_NONE; MHAQ_FQ_ACT_RELU: t unchanged if NaN, else fmaxf(t, 0) (torch's
+ *                CUDA relu); MHAQ_FQ_ACT_LEAKY_RELU: t > 0 ? t : t * negative_slope (fp32);
+ *   and writes any non-empty combination of
+ *     y          fp32 [m][n_out], or NULL;
+ *     codes      uint8 [m][cp_out], cp_out = round_up(n_out, 16), 16-byte aligned, or NULL: the
+ *                forward's code of t under the next quantizer's per-tensor LINEAR operands
+ *                (code_scale, code_zero_point, code_max_val; one float each), exactly as
+ *                mhaq_fq_act_codes_f32 forms it, saturated to [0, 255] (NaN -> 0), not counted;
+ *                channels [n_out, cp_out) are 0. */
+#define MHAQ_FQ_ACT_NONE 0
+#define MHAQ_FQ_ACT_RELU 1
+#define MHAQ_FQ_ACT_LEAKY_RELU 2
+
+typedef struct mhaq_fq_iconv_epilogue {
+    const float *residual;
+    int activation;
+    float negative_slope;
+    float *y;
+    uint8_t *codes;
+    const float *code_scale;
+    const float *code_zero_point;
+    const float *code_max_val;
+} mhaq_fq_iconv_epilogue;
+
+/* mhaq_fq_iconv_u8's arguments without y, plus the epilogue above.  Errors (before any CUDA call):
+ * those of mhaq_fq_iconv_u8, no output, codes without all three code operands, an unknown
+ * activation and a misaligned codes buffer.  Capture-safe like mhaq_fq_iconv_u8. */
+int mhaq_fq_iconv_fused_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                           const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                           int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
+                           int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                           int act_max_code, int weight_max_code, const mhaq_fq_iconv_epilogue *epilogue,
+                           void *stream);
 
 #ifdef __cplusplus
 }

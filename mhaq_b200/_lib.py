@@ -30,6 +30,15 @@ class WRowBwdDesc(ctypes.Structure):
         ("n_rows", c_int64), ("n_inner", c_int64), ("g_log_scale_acc", c_void_p)]
 
 
+class IConvEpilogue(ctypes.Structure):
+    """mhaq_fq_iconv_epilogue"""
+    _fields_ = [("residual", c_void_p), ("activation", c_int), ("negative_slope", c_float), ("y", c_void_p),
+                ("codes", c_void_p), ("code_scale", c_void_p), ("code_zero_point", c_void_p),
+                ("code_max_val", c_void_p)]
+
+
+ACT_NONE, ACT_RELU, ACT_LEAKY_RELU = 0, 1, 2  # MHAQ_FQ_ACT_*
+
 # name -> (restype, argtypes); mirrors include/mhaq_fq.h one to one
 _P = c_void_p
 _SIGNATURES = {
@@ -78,6 +87,8 @@ _SIGNATURES = {
     "mhaq_fq_act_codes_f32": (c_int, [_P, _P, _P, _P, _P, c_int64, c_int64, c_int64, _P, _P]),
     "mhaq_fq_iconv_u8": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, _P, c_int64, c_int64, c_int64, c_int64,
                                  c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P]),
+    "mhaq_fq_iconv_fused_u8": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int64, c_int64, c_int64, c_int64,
+                                       c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

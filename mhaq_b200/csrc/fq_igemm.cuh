@@ -175,8 +175,99 @@ struct IConvArgs {
     int64_t m, h, w, cp, n_out, ho, wo, k_chunks, k_stages;
     int kh, kw, sh, sw, ph, pw, n_wcls, tile_n, tile_out, tmem_cols;
     int vec_out;               // y 16-byte aligned and n_out % 4 == 0: float4 stores
+    // fused epilogue (fq_iconv_kernel<true> only)
+    const float *res;          // residual [m][n_out] or NULL
+    uint8_t *codes;            // next layer's codes [m][cp_out] or NULL (y may then be NULL)
+    const float *code_s, *code_zp, *code_hi;   // its per-tensor LINEAR operands
+    int64_t cp_out;
+    float slope;               // LeakyReLU negative slope
+    int act;                   // kIcAct*
+    int vec_res;               // res 16-byte aligned and n_out % 4 == 0: float4 loads
 };
 
+constexpr int kIcActNone = 0, kIcActRelu = 1, kIcActLeaky = 2;   // = MHAQ_FQ_ACT_*
+
+// Fused epilogue of one 16-column chunk: t = out (+ residual), activation, then fp32 and / or the
+// next layer's codes.  relu keeps NaN and is fmaxf(t, 0) otherwise, as torch's CUDA clamp_min;
+// LeakyReLU is t > 0 ? t : t * slope, as torch's CUDA leaky_relu.  The codes are the forward's
+// rint(v) of t exactly as fq_act_codes_kernel forms them (fwd_pair_fast where its guard allows it,
+// fwd_elem otherwise: bit-identical), saturated to [0, 255] with NaN -> 0 and not counted.
+// The residual of a chunk, loaded before its accumulator columns are read so that the two
+// latencies overlap (0 where nv or the row ends).
+__device__ __forceinline__ void iconv_load_res(const IConvArgs &p, float (&r)[16], int64_t m, int64_t n0, int nv) {
+    const float *rrow = p.res + m * p.n_out + n0;
+    if (p.vec_res && (n0 & 3) == 0 && nv == 16) {
+#pragma unroll
+        for (int i = 0; i < 16; i += 4) {
+            const float4 v = __ldg(reinterpret_cast<const float4 *>(rrow + i));
+            r[i] = v.x; r[i + 1] = v.y; r[i + 2] = v.z; r[i + 3] = v.w;
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) r[i] = i < nv ? __ldg(rrow + i) : 0.f;
+    }
+}
+
+__device__ __forceinline__ void iconv_fused_chunk(const IConvArgs &p, float (&out)[16], const float (&r)[16],
+                                                  int64_t m, int64_t n0, int nv, bool vec, const QConst &q,
+                                                  const Div2 &dv, f32x2 zpn, f32x2 zp2, bool fast_ok) {
+    if (p.res) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) out[i] = __fadd_rn(out[i], r[i]);
+    }
+    if (p.act == kIcActRelu) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) out[i] = isnan(out[i]) ? out[i] : fmaxf(out[i], 0.f);
+    } else if (p.act == kIcActLeaky) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) out[i] = out[i] > 0.f ? out[i] : __fmul_rn(out[i], p.slope);
+    }
+    if (p.y) {
+        float *yrow = p.y + m * p.n_out + n0;
+        if (vec && nv == 16) {
+#pragma unroll
+            for (int i = 0; i < 16; i += 4)
+                *reinterpret_cast<float4 *>(yrow + i) = make_float4(out[i], out[i + 1], out[i + 2], out[i + 3]);
+        } else {
+#pragma unroll
+            for (int i = 0; i < 16; ++i)
+                if (i < nv) yrow[i] = out[i];
+        }
+    }
+    if (p.codes) {
+        uint32_t c[16], bad = 0;
+#pragma unroll
+        for (int i = 0; i < 16; i += 2) {
+            float c0, c1, y0, y1;
+            if (fast_ok && !(fmaxf(fabsf(out[i]), fabsf(out[i + 1])) > kXHi)) {
+                fwd_pair_fast<true>(out[i], out[i + 1], q, dv, zpn, zp2, y0, y1, c0, c1);
+            } else {
+                (void)fwd_elem(out[i], q, c0);
+                (void)fwd_elem(out[i + 1], q, c1);
+            }
+            c[i] = sat_code<8>(c0, bad);
+            c[i + 1] = sat_code<8>(c1, bad);
+        }
+        uint8_t *crow = p.codes + m * p.cp_out + n0;
+        if (nv == 16 && (n0 & 15) == 0) {
+            uint4 w;
+            w.x = (uint32_t)pack4<8>(c[0], c[1], c[2], c[3]);
+            w.y = (uint32_t)pack4<8>(c[4], c[5], c[6], c[7]);
+            w.z = (uint32_t)pack4<8>(c[8], c[9], c[10], c[11]);
+            w.w = (uint32_t)pack4<8>(c[12], c[13], c[14], c[15]);
+            *reinterpret_cast<uint4 *>(crow) = w;
+        } else {
+#pragma unroll
+            for (int i = 0; i < 16; ++i)
+                if (i < nv) crow[i] = (uint8_t)c[i];
+        }
+    }
+}
+
+// FUSED = false: y = alpha * S + beta * SA + C, fp32 only (mhaq_fq_iconv_u8).  FUSED = true: the
+// same value through iconv_fused_chunk (mhaq_fq_iconv_fused_u8); the tile holding the last output
+// channels also writes the codes' padding channels [n_out, cp_out) as 0.
+template <bool FUSED>
 __global__ void __launch_bounds__(kIcThreads, 1)
 fq_iconv_kernel(const IConvArgs p) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -283,8 +374,26 @@ fq_iconv_kernel(const IConvArgs p) {
         const int64_t n_here = (p.n_out - n_base) < p.tile_out ? (p.n_out - n_base) : p.tile_out;
         float *yrow = p.y + m * p.n_out + n_base;
         const bool vec = p.vec_out && (n_base & 3) == 0;
+        QConst cq{};
+        Div2 cdv{};
+        f32x2 czpn{}, czp2{};
+        bool cfast = false;
+        if constexpr (FUSED) {
+            if (p.codes) {
+                const QParams prm = {p.code_s, p.code_zp, p.code_zp, p.code_hi, 0, 0, 0, 0, PARAMS_LINEAR};
+                cq = load_qconst(prm, 0);
+                cdv = make_div2(cq.s, __frcp_rn(cq.s));
+                czpn = bc2(-cq.zp);
+                czp2 = bc2(cq.zp);
+                cfast = scale_fast_ok(cq.s);
+            }
+        }
         for (int col = 0; col < n_here; col += 16) {
             uint32_t v[16];
+            [[maybe_unused]] float rv[16];
+            if constexpr (FUSED) {
+                if (p.res && live) iconv_load_res(p, rv, m, n_base + col, n_here - col < 16 ? (int)(n_here - col) : 16);
+            }
             tmem_ld16(lane_addr + col, v);
             tmem_wait_ld();
             if (!live) continue;
@@ -300,7 +409,10 @@ fq_iconv_kernel(const IConvArgs p) {
                     out[i] = 0.f;
                 }
             }
-            if (vec && col + 16 <= n_here) {
+            if constexpr (FUSED) {
+                const int nv = n_here - col < 16 ? (int)(n_here - col) : 16;
+                iconv_fused_chunk(p, out, rv, m, n_base + col, nv, vec, cq, cdv, czpn, czp2, cfast);
+            } else if (vec && col + 16 <= n_here) {
 #pragma unroll
                 for (int i = 0; i < 16; i += 4)
                     *reinterpret_cast<float4 *>(yrow + col + i) = make_float4(out[i], out[i + 1], out[i + 2], out[i + 3]);
@@ -309,6 +421,10 @@ fq_iconv_kernel(const IConvArgs p) {
                 for (int i = 0; i < 16; ++i)
                     if (col + i < n_here) yrow[col + i] = out[i];
             }
+        }
+        if constexpr (FUSED) {
+            if (p.codes && live && tile == (int)gridDim.y - 1)
+                for (int64_t n = p.n_out; n < p.cp_out; ++n) p.codes[m * p.cp_out + n] = 0;
         }
     } else if (tid == 128) {
         // ---------------- MMA issuer ----------------

@@ -1787,17 +1787,59 @@ void launch_unpack(bool vec, int grid, cudaStream_t st, const uint8_t *packed, f
 }
 
 // ---- integer layers (fq_igemm.cuh) ----
-// The iconv kernel needs more than 48 KiB of dynamic shared memory: opt in once per device.
+// The iconv kernel needs more than 48 KiB of dynamic shared memory: opt in once per device and
+// instantiation.
+template <bool FUSED>
 inline int iconv_smem_opt_in() {
     static bool done[64] = {};
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return (int)e;
     if (dev < 64 && done[dev]) return 0;
-    e = cudaFuncSetAttribute(fq_iconv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    e = cudaFuncSetAttribute(fq_iconv_kernel<FUSED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)iconv_smem_bytes(kIcMaxTileN));
     if (e != cudaSuccess) return (int)e;
     if (dev < 64) done[dev] = true;
+    return 0;
+}
+
+// Argument checks and kernel arguments shared by mhaq_fq_iconv_u8 and mhaq_fq_iconv_fused_u8 (no
+// CUDA call); the epilogue fields of `a` are left zero and y to the caller.
+inline int iconv_args(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                      const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                      int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out, int kernel_h,
+                      int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int act_max_code,
+                      int weight_max_code, IConvArgs &a, dim3 &grid) {
+    if (!codes || !weights || !alpha || !beta || !ctab || !h_class || !w_class) return MHAQ_FQ_ENULL;
+    if (batch < 1 || height < 1 || width < 1 || cp < 16 || cp % 16 != 0 || n_out < 1 || n_w_classes < 1)
+        return MHAQ_FQ_EINVAL;
+    if (kernel_h < 1 || kernel_w < 1 || stride_h < 1 || stride_w < 1 || pad_h < 0 || pad_w < 0)
+        return MHAQ_FQ_EINVAL;
+    if (act_max_code < 1 || act_max_code > 255 || weight_max_code < 1 || weight_max_code > 255)
+        return MHAQ_FQ_EINVAL;
+    if (!aligned16(codes) || !aligned16(weights)) return MHAQ_FQ_EINVAL;
+    const int64_t ho = (height + 2 * pad_h - kernel_h) / stride_h + 1;
+    const int64_t wo = (width + 2 * pad_w - kernel_w) / stride_w + 1;
+    if (height + 2 * pad_h < kernel_h || width + 2 * pad_w < kernel_w) return MHAQ_FQ_EINVAL;
+    const int64_t k_bytes = (int64_t)kernel_h * kernel_w * cp;
+    // the int32 accumulator holds sum_k ca_k * cw_nk <= K * act_max_code * weight_max_code
+    if (k_bytes > (int64_t)1 << 31 || k_bytes * act_max_code * weight_max_code >= ((int64_t)1 << 31))
+        return MHAQ_FQ_EINVAL;
+    const IcLayout l = iconv_layout(n_out, k_bytes);
+    if (l.tile_n > kIcMaxTileN) return MHAQ_FQ_EINVAL;
+    const int64_t m = batch * ho * wo;
+    const int64_t m_tiles = (m + kIcTileM - 1) / kIcTileM;
+    if (m_tiles > 0x7fffffffLL) return MHAQ_FQ_EINVAL;
+    a = IConvArgs{};
+    a.a = codes; a.b = weights; a.alpha = alpha; a.beta = beta; a.ctab = ctab;
+    a.hcls = h_class; a.wcls = w_class;
+    a.m = m; a.h = height; a.w = width; a.cp = cp; a.n_out = n_out; a.ho = ho; a.wo = wo;
+    a.k_chunks = k_bytes / 16; a.k_stages = l.k_stages;
+    a.kh = kernel_h; a.kw = kernel_w; a.sh = stride_h; a.sw = stride_w; a.ph = pad_h; a.pw = pad_w;
+    a.n_wcls = n_w_classes; a.tile_n = l.tile_n; a.tile_out = l.tile_out;
+    a.tmem_cols = 32;
+    while (a.tmem_cols < l.tile_n) a.tmem_cols <<= 1;
+    grid = dim3((unsigned)m_tiles, (unsigned)l.n_tiles);
     return 0;
 }
 
@@ -2353,40 +2395,53 @@ int mhaq_fq_iconv_u8(const uint8_t *codes, const uint8_t *weights, const float *
                      float *y, int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
                      int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                      int act_max_code, int weight_max_code, void *stream) {
-    if (!codes || !weights || !alpha || !beta || !ctab || !h_class || !w_class || !y) return MHAQ_FQ_ENULL;
-    if (batch < 1 || height < 1 || width < 1 || cp < 16 || cp % 16 != 0 || n_out < 1 || n_w_classes < 1)
-        return MHAQ_FQ_EINVAL;
-    if (kernel_h < 1 || kernel_w < 1 || stride_h < 1 || stride_w < 1 || pad_h < 0 || pad_w < 0)
-        return MHAQ_FQ_EINVAL;
-    if (act_max_code < 1 || act_max_code > 255 || weight_max_code < 1 || weight_max_code > 255)
-        return MHAQ_FQ_EINVAL;
-    if (!aligned16(codes) || !aligned16(weights)) return MHAQ_FQ_EINVAL;
-    const int64_t ho = (height + 2 * pad_h - kernel_h) / stride_h + 1;
-    const int64_t wo = (width + 2 * pad_w - kernel_w) / stride_w + 1;
-    if (height + 2 * pad_h < kernel_h || width + 2 * pad_w < kernel_w) return MHAQ_FQ_EINVAL;
-    const int64_t k_bytes = (int64_t)kernel_h * kernel_w * cp;
-    // the int32 accumulator holds sum_k ca_k * cw_nk <= K * act_max_code * weight_max_code
-    if (k_bytes > (int64_t)1 << 31 || k_bytes * act_max_code * weight_max_code >= ((int64_t)1 << 31))
-        return MHAQ_FQ_EINVAL;
-    const IcLayout l = iconv_layout(n_out, k_bytes);
-    if (l.tile_n > kIcMaxTileN) return MHAQ_FQ_EINVAL;
-    const int64_t m = batch * ho * wo;
-    const int64_t m_tiles = (m + kIcTileM - 1) / kIcTileM;
-    if (m_tiles > 0x7fffffffLL) return MHAQ_FQ_EINVAL;
-    int rc = iconv_smem_opt_in();
-    if (rc) return rc;
+    if (!y) return MHAQ_FQ_ENULL;
     IConvArgs a;
-    a.a = codes; a.b = weights; a.alpha = alpha; a.beta = beta; a.ctab = ctab;
-    a.hcls = h_class; a.wcls = w_class; a.y = y;
-    a.m = m; a.h = height; a.w = width; a.cp = cp; a.n_out = n_out; a.ho = ho; a.wo = wo;
-    a.k_chunks = k_bytes / 16; a.k_stages = l.k_stages;
-    a.kh = kernel_h; a.kw = kernel_w; a.sh = stride_h; a.sw = stride_w; a.ph = pad_h; a.pw = pad_w;
-    a.n_wcls = n_w_classes; a.tile_n = l.tile_n; a.tile_out = l.tile_out;
-    a.tmem_cols = 32;
-    while (a.tmem_cols < l.tile_n) a.tmem_cols <<= 1;
+    dim3 grid;
+    int rc = iconv_args(codes, weights, alpha, beta, ctab, h_class, w_class, n_w_classes, batch, height, width, cp,
+                        n_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, act_max_code, weight_max_code,
+                        a, grid);
+    if (rc) return rc;
+    rc = iconv_smem_opt_in<false>();
+    if (rc) return rc;
+    a.y = y;
     a.vec_out = aligned16(y) && n_out % 4 == 0;
-    const dim3 grid((unsigned)m_tiles, (unsigned)l.n_tiles);
-    fq_iconv_kernel<<<grid, kIcThreads, iconv_smem_bytes(l.tile_n), (cudaStream_t)stream>>>(a);
+    fq_iconv_kernel<false><<<grid, kIcThreads, iconv_smem_bytes(a.tile_n), (cudaStream_t)stream>>>(a);
+    return last_error();
+}
+
+int mhaq_fq_iconv_fused_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                           const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                           int64_t batch, int64_t height, int64_t width, int64_t cp, int64_t n_out,
+                           int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                           int act_max_code, int weight_max_code, const mhaq_fq_iconv_epilogue *epilogue,
+                           void *stream) {
+    if (!epilogue) return MHAQ_FQ_ENULL;
+    const mhaq_fq_iconv_epilogue &e = *epilogue;
+    if (!e.y && !e.codes) return MHAQ_FQ_EINVAL;
+    if (e.codes && (!e.code_scale || !e.code_zero_point || !e.code_max_val)) return MHAQ_FQ_ENULL;
+    if (e.codes && !aligned16(e.codes)) return MHAQ_FQ_EINVAL;
+    if (e.activation != MHAQ_FQ_ACT_NONE && e.activation != MHAQ_FQ_ACT_RELU &&
+        e.activation != MHAQ_FQ_ACT_LEAKY_RELU)
+        return MHAQ_FQ_EINVAL;
+    IConvArgs a;
+    dim3 grid;
+    int rc = iconv_args(codes, weights, alpha, beta, ctab, h_class, w_class, n_w_classes, batch, height, width, cp,
+                        n_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, act_max_code, weight_max_code,
+                        a, grid);
+    if (rc) return rc;
+    rc = iconv_smem_opt_in<true>();
+    if (rc) return rc;
+    a.y = e.y;
+    a.vec_out = e.y && aligned16(e.y) && n_out % 4 == 0;
+    a.res = e.residual;
+    a.vec_res = e.residual && aligned16(e.residual) && n_out % 4 == 0;
+    a.act = e.activation;
+    a.slope = e.negative_slope;
+    a.codes = e.codes;
+    a.code_s = e.code_scale; a.code_zp = e.code_zero_point; a.code_hi = e.code_max_val;
+    a.cp_out = (n_out + 15) / 16 * 16;
+    fq_iconv_kernel<true><<<grid, kIcThreads, iconv_smem_bytes(a.tile_n), (cudaStream_t)stream>>>(a);
     return last_error();
 }
 

@@ -10,12 +10,14 @@ from __future__ import annotations
 
 import ctypes
 import math
+import dataclasses
 from dataclasses import dataclass
 from typing import Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
 
+from . import _lib
 from ._lib import lib, check
 
 _check_rc = check   # for functions whose `check` argument shadows it
@@ -1287,10 +1289,26 @@ class IntLayerOperands:
     zpa: float
     bias: Optional[torch.Tensor]  # fp64 [N] or None
     tables: dict
+    sa: float                     # activation scale
 
     @property
     def cp(self) -> int:
         return code_channels(self.cin)
+
+    def fold_affine(self, k, shift) -> "IntLayerOperands":
+        """Operands of ``k * y + shift`` (``k``, ``shift``: ``[N]``, taken in fp64), e.g. an eval
+        BatchNorm after the layer: sw, zpw and bias become ``k * sw``, ``k * zpw`` and
+        ``k * bias + shift`` in fp64, so alpha = RN32(sa * k * sw), beta = RN32(sa * k * zpw) and
+        every constant-table entry RN32(k * C64 + shift) are formed from the fp64 terms and rounded
+        once (DESIGN §3, "Fused epilogue").  Shares the weight operand; the pattern tables are
+        rebuilt on first use."""
+        f64 = dict(dtype=torch.float64, device=self.sw.device)
+        k = torch.as_tensor(k).to(**f64).reshape(-1).expand(self.n_out)
+        shift = torch.as_tensor(shift).to(**f64).reshape(-1).expand(self.n_out)
+        sw, zpw = k * self.sw, k * self.zpw
+        bias = shift.clone() if self.bias is None else k * self.bias + shift
+        return dataclasses.replace(self, alpha=(self.sa * sw).float(), beta=(self.sa * zpw).float(), sw=sw,
+                                   zpw=zpw, bias=bias, tables={})
 
     def constant_table(self, hvalid: torch.Tensor, wvalid: torch.Tensor) -> torch.Tensor:
         """fp64 ctab [n_h_classes * n_w_classes][N]: zpa * (sw * sum_{k in p} cw + zpw * |p|) + bias."""
@@ -1342,7 +1360,30 @@ def int_layer_operands(cw, sw, zpw, sa, zpa, bias, a_top: int, w_top: int) -> In
         n_out=n, cin=c, kh=kh, kw=kw, a_top=a_top, w_top=w_top,
         tap_sums=cw.to(**f64).sum(1), sw=sw, zpw=zpw, zpa=zpa,
         bias=None if bias is None else torch.as_tensor(bias).to(**f64).reshape(n),
-        tables={})
+        tables={}, sa=sa)
+
+
+def batchnorm_foldable(bn) -> bool:
+    """An eval-mode ``BatchNorm2d`` that normalizes with its running statistics."""
+    return (isinstance(bn, torch.nn.BatchNorm2d) and not bn.training and bn.track_running_stats
+            and bn.running_mean is not None and bn.running_var is not None)
+
+
+def fold_batchnorm(L: IntLayerOperands, bn) -> IntLayerOperands:
+    """``L`` followed by the eval BatchNorm ``bn``: ``IntLayerOperands.fold_affine`` with
+    k = gamma / sqrt(running_var + eps) and shift = beta - k * running_mean, all in fp64
+    (``affine=False``: gamma = 1, beta = 0).  A BatchNorm without running statistics (or in
+    training mode) normalizes with the batch's statistics and cannot be folded: ValueError."""
+    if not batchnorm_foldable(bn):
+        raise ValueError("fold_batchnorm: only an eval-mode BatchNorm2d with running statistics can be folded")
+    if bn.num_features != L.n_out:
+        raise ValueError(f"fold_batchnorm: {bn.num_features} BatchNorm features for {L.n_out} output channels")
+    f64 = dict(dtype=torch.float64, device=L.sw.device)
+    var, mean = bn.running_var.detach().to(**f64), bn.running_mean.detach().to(**f64)
+    gamma = bn.weight.detach().to(**f64) if bn.affine else torch.ones_like(var)
+    b = bn.bias.detach().to(**f64) if bn.affine else torch.zeros_like(var)
+    k = gamma / torch.sqrt(var + float(bn.eps))
+    return L.fold_affine(k, b - k * mean)
 
 
 def _iconv(codes, L: IntLayerOperands, y, b, h, w, stride, padding):
@@ -1372,6 +1413,57 @@ def int_conv2d(codes, L: IntLayerOperands, stride=1, padding=0) -> torch.Tensor:
     y = torch.empty((b, L.n_out, ho, wo), dtype=torch.float32, device=codes.device,
                     memory_format=torch.channels_last)
     return _iconv(codes, L, y, b, h, w, stride, padding)
+
+
+ACTIVATIONS = {None: _lib.ACT_NONE, "relu": _lib.ACT_RELU, "leaky_relu": _lib.ACT_LEAKY_RELU}
+
+
+def int_conv2d_fused(codes, L: IntLayerOperands, stride=1, padding=0, *, residual=None, activation=None,
+                     negative_slope=None, out_fp32=True, code_params=None):
+    """``int_conv2d`` with its epilogue extended (mhaq_fq_iconv_fused_u8): t = the convolution
+    (with whatever ``fold_batchnorm`` folded into ``L``), then ``t + residual`` (fp32, the output's
+    shape; made channels_last-contiguous, which copies an NCHW tensor), then ``activation``
+    (None, "relu" or "leaky_relu" with ``negative_slope``, default 0.01), one launch.  Returns
+    ``(y, codes)``: y the channels_last fp32 ``[B, N, Ho, Wo]`` if ``out_fp32``, codes the uint8
+    ``[B, Ho, Wo, code_channels(N)]`` of the next ``NoisyAct`` if ``code_params`` = (scale,
+    zero_point, max_val) is given (as ``act_codes`` would make them from y), else None."""
+    if activation not in ACTIVATIONS:
+        raise ValueError(f"int_conv2d_fused: unknown activation {activation!r}")
+    if not out_fp32 and code_params is None:
+        raise ValueError("int_conv2d_fused: no output requested")
+    b, h, w, _ = codes.shape
+    stride, padding = _pair(stride), _pair(padding)
+    ho = (h + 2 * padding[0] - L.kh) // stride[0] + 1
+    wo = (w + 2 * padding[1] - L.kw) // stride[1] + 1
+    dev = codes.device
+    y = torch.empty((b, L.n_out, ho, wo), dtype=torch.float32, device=dev,
+                    memory_format=torch.channels_last) if out_fp32 else None
+    out_codes, prm = None, (None, None, None)
+    if code_params is not None:
+        out_codes = torch.empty((b, ho, wo, code_channels(L.n_out)), dtype=torch.uint8, device=dev)
+        prm = tuple(torch.as_tensor(p).to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+                    for p in code_params)
+        if len(prm) != 3:
+            raise ValueError("int_conv2d_fused: code_params is (scale, zero_point, max_val)")
+    if residual is not None:
+        if (residual.dtype != torch.float32 or tuple(residual.shape) != (b, L.n_out, ho, wo)
+                or residual.device != dev):
+            raise ValueError(f"int_conv2d_fused: the residual must be fp32 {(b, L.n_out, ho, wo)} on {dev}, "
+                             f"got {residual.dtype} {tuple(residual.shape)} on {residual.device}")
+        residual = residual.detach().contiguous(memory_format=torch.channels_last)
+    hc, wc, nwc, ctab = L.pattern_tables(h, w, stride, padding)
+    if codes.shape[-1] != L.cp or codes.dtype != torch.uint8 or not codes.is_contiguous():
+        raise ValueError(f"integer layer: expected contiguous uint8 codes with {L.cp} channels, "
+                         f"got {codes.dtype} {tuple(codes.shape)}")
+    if b * ho * wo:
+        slope = 0.01 if negative_slope is None else float(negative_slope)
+        epi = _lib.IConvEpilogue(_ptr(residual), ACTIVATIONS[activation], slope, _ptr(y), _ptr(out_codes),
+                                 *(_ptr(p) for p in prm))
+        _check_rc(lib.mhaq_fq_iconv_fused_u8(_ptr(codes), _ptr(L.weight), _ptr(L.alpha), _ptr(L.beta), _ptr(ctab),
+                                             _ptr(hc), _ptr(wc), nwc, b, h, w, L.cp, L.n_out, L.kh, L.kw,
+                                             stride[0], stride[1], padding[0], padding[1], L.a_top, L.w_top,
+                                             ctypes.byref(epi), _stream()), "mhaq_fq_iconv_fused_u8")
+    return y, out_codes
 
 
 def int_linear(codes, L: IntLayerOperands) -> torch.Tensor:

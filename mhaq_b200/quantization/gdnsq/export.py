@@ -182,3 +182,4 @@ def load_quantized(model, blob) -> None:
 
 
 from .inference import build_integer_model  # noqa: E402,F401  (runs an export on its integer codes)
+from .inference import fuse_integer_model  # noqa: E402,F401  (fuses BN / add / activation / codes into it)
