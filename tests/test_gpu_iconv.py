@@ -88,8 +88,10 @@ def test_act_codes_equal_packed_8bit_codes(c):
 # operator bar against the fp64 convolution of the exact dequantized values
 # ---------------------------------------------------------------------------------------------
 def _random_layer(n, c, k, w_bits, levels, per_channel, bias, signed, seed):
+    """Random operands of an n x c layer with kernel ``k`` = (kh, kw) (or one int for k x k)."""
+    kh, kw = (k, k) if isinstance(k, int) else k
     g = torch.Generator(device=DEV).manual_seed(seed)
-    cw = torch.randint(0, 1 << w_bits, (n, c, k, k), generator=g, device=DEV)
+    cw = torch.randint(0, 1 << w_bits, (n, c, kh, kw), generator=g, device=DEV)
     rows = n if per_channel else 1
     sw = torch.exp2(torch.randint(-10, -4, (rows,), generator=g, device=DEV).float()
                     + torch.rand(rows, generator=g, device=DEV))
@@ -102,17 +104,18 @@ def _random_layer(n, c, k, w_bits, levels, per_channel, bias, signed, seed):
 
 
 def _check_bar(y, codes_nchw, L, cw, sw, zpw, sa, zpa, b, stride, pad):
-    """|y - ref64| <= 4u (|alpha S| + |beta SA| + |C|), the terms exact (integer sums in int64)."""
-    n, c, k, _ = cw.shape
+    """|y - ref64| <= 4u (|alpha S| + |beta SA| + |C|), the terms exact (integer sums in int64).
+    ``stride`` and ``pad`` are (h, w) pairs."""
+    n, c, kh, kw = cw.shape
     ca = codes_nchw.double()
     a = ca * sa + zpa
     wt = cw.double() * sw.double().reshape(-1, 1, 1, 1) + zpw.double().reshape(-1, 1, 1, 1)
     ref = F.conv2d(a, wt, None if b is None else b.double(), stride=stride, padding=pad)
     s = F.conv2d(ca, cw.double(), stride=stride, padding=pad).round().long()
-    sa_m = F.conv2d(ca, torch.ones(1, c, k, k, dtype=torch.float64, device=DEV), stride=stride,
+    sa_m = F.conv2d(ca, torch.ones(1, c, kh, kw, dtype=torch.float64, device=DEV), stride=stride,
                     padding=pad).round().long()
     h, w = codes_nchw.shape[2:]
-    hc, wc, nwc, ctab = L.pattern_tables(h, w, (stride, stride), (pad, pad))
+    hc, wc, nwc, ctab = L.pattern_tables(h, w, stride, pad)
     p = hc.long()[:, None] * nwc + wc.long()[None, :]
     cterm = ctab.double()[p].permute(2, 0, 1)[None]
     terms = ((L.alpha.double().reshape(1, -1, 1, 1) * s.double()).abs()
@@ -124,17 +127,33 @@ def _check_bar(y, codes_nchw, L, cw, sw, zpw, sa, zpa, b, stride, pad):
     assert bool(ok.all()), f"max err / bar {float((err / (4 * U * terms)).max()):.3g}"
 
 
-OP_CASES = [  # (B, H, W, C, N, k, stride, pad, w_bits, levels)
-    (2, 9, 7, 3, 10, 3, 1, 1, 4, 16),
-    (3, 11, 11, 8, 16, 3, 2, 1, 2, 4),
-    (2, 16, 16, 12, 48, 3, 2, 0, 8, 256),
-    (4, 8, 8, 16, 64, 3, 1, 1, 1, 2),
-    (2, 13, 10, 50, 64, 3, 1, 1, 4, 16),
-    (1, 9, 9, 64, 512, 3, 2, 1, 4, 3),
-    (2, 5, 6, 512, 48, 3, 1, 1, 8, 256),
-    (3, 10, 10, 12, 16, 1, 1, 0, 2, 200),
-    (2, 7, 7, 16, 10, 7, 2, 3, 4, 16),
-    (2, 6, 6, 16, 511, 3, 1, 1, 4, 16),          # 511 = 2 * 255 + 1: three weight tiles
+OP_CASES = [  # (B, H, W, C, N, (kh, kw), (sh, sw), (ph, pw), w_bits, levels)
+    (2, 9, 7, 3, 10, (3, 3), (1, 1), (1, 1), 4, 16),
+    (3, 11, 11, 8, 16, (3, 3), (2, 2), (1, 1), 2, 4),
+    (2, 16, 16, 12, 48, (3, 3), (2, 2), (0, 0), 8, 256),
+    (4, 8, 8, 16, 64, (3, 3), (1, 1), (1, 1), 1, 2),
+    (2, 13, 10, 50, 64, (3, 3), (1, 1), (1, 1), 4, 16),
+    (1, 9, 9, 64, 512, (3, 3), (2, 2), (1, 1), 4, 3),
+    (2, 5, 6, 512, 48, (3, 3), (1, 1), (1, 1), 8, 256),
+    (3, 10, 10, 12, 16, (1, 1), (1, 1), (0, 0), 2, 200),
+    (2, 7, 7, 16, 10, (7, 7), (2, 2), (3, 3), 4, 16),
+    (2, 6, 6, 16, 511, (3, 3), (1, 1), (1, 1), 4, 16),          # 511 = 2 * 255 + 1: three weight tiles
+    # per-axis geometry: every axis pair differs, so a swapped kh / kw, sh / sw or ph / pw fails
+    (2, 9, 12, 16, 24, (1, 3), (1, 2), (0, 1), 4, 16),
+    (2, 10, 7, 8, 20, (3, 1), (1, 1), (1, 0), 2, 4),
+    (2, 13, 14, 5, 33, (5, 3), (1, 3), (0, 0), 4, 16),
+    (2, 15, 9, 12, 40, (7, 3), (2, 1), (3, 0), 8, 256),
+    (3, 8, 8, 16, 16, (2, 2), (1, 1), (0, 0), 4, 16),          # even kernels
+    (2, 9, 10, 24, 18, (2, 4), (2, 1), (1, 2), 4, 16),
+    (2, 12, 13, 16, 16, (2, 3), (3, 4), (1, 0), 4, 16),        # stride larger than the kernel
+    # degenerate windows: pad >= k gives rows / columns with no valid tap (C alone)
+    (2, 2, 2, 16, 12, (3, 3), (1, 1), (3, 3), 4, 16),          # image smaller than the kernel
+    (2, 5, 6, 16, 20, (1, 1), (1, 1), (1, 1), 4, 16),
+    (3, 1, 1, 16, 24, (3, 3), (1, 1), (4, 1), 4, 16),          # 1 x 1 image, 7 x 1 output
+    (2, 11, 10, 16, 32, (1, 1), (3, 2), (0, 0), 4, 16),
+    (4, 14, 14, 64, 128, (1, 1), (2, 2), (0, 0), 4, 16),       # ResNet downsample
+    (3, 5, 7, 16, 40, (5, 7), (1, 1), (0, 0), 4, 16),          # kernel = image: 1 x 1 output
+    (5, 1, 1, 32, 48, (1, 1), (1, 1), (0, 0), 4, 16),          # H = W = 1
 ]
 
 
@@ -163,7 +182,7 @@ def test_int_linear_operator_bar(bsz, c, n, w_bits, levels):
     codes[:, :c] = ca.to(torch.uint8)
     y = ops.int_linear(codes, L)
     assert y.shape == (bsz, n)
-    _check_bar(y[:, :, None, None], ca[:, :, None, None], L, cw, sw, zpw, sa, zpa, b, 1, 0)
+    _check_bar(y[:, :, None, None], ca[:, :, None, None], L, cw, sw, zpw, sa, zpa, b, (1, 1), (0, 0))
 
 
 def test_more_than_2p31_outputs():
@@ -177,7 +196,7 @@ def test_more_than_2p31_outputs():
     rows = torch.cat([torch.arange(0, 3000, device=DEV), torch.arange(m - 3000, m, device=DEV),
                       torch.randint(0, m, (3000,), device=DEV)])
     ca = codes[rows, :c].long()
-    _check_bar(y[rows][:, :, None, None], ca[:, :, None, None], L, cw, sw, zpw, sa, zpa, b, 1, 0)
+    _check_bar(y[rows][:, :, None, None], ca[:, :, None, None], L, cw, sw, zpw, sa, zpa, b, (1, 1), (0, 0))
     del y, codes
     torch.cuda.empty_cache()
 
@@ -186,7 +205,7 @@ def test_more_than_2p31_outputs():
 # exported models
 # ---------------------------------------------------------------------------------------------
 MODELS = [("resnet20", "STE", False), ("resnet20", "LSQ", False), ("resnet20", "STE", True),
-          ("resnet20_per_tensor", "LSQ", False), ("bias_net", "STE", False)]
+          ("resnet20_per_tensor", "LSQ", False), ("bias_net", "STE", False), ("asym_net", "STE", False)]
 
 
 def _trained(kind, method, channels_last):

@@ -67,7 +67,7 @@ def test_epilogue_equals_composition(ci, residual, activation, outputs):
     codes = torch.zeros(bsz, h, w, L.cp, dtype=torch.uint8, device=DEV)
     codes[..., :c] = ca.permute(0, 2, 3, 1).to(torch.uint8)
     # channel 0 gives t = -0 exactly: alpha = beta = -0 and C = -0 (fma(-0, x, -0) = -0)
-    hc, wc, nwc, ctab = L.pattern_tables(h, w, (stride, stride), (pad, pad))
+    hc, wc, nwc, ctab = L.pattern_tables(h, w, stride, pad)
     L.alpha[0], L.beta[0] = -0.0, -0.0
     ctab[:, 0] = -0.0
     plain = ops.int_conv2d(codes, L, stride, pad)
@@ -146,7 +146,8 @@ def _rfdn():
 
 
 MODELS = [("resnet20", "STE", False), ("resnet20", "LSQ", False), ("resnet20", "STE", True),
-          ("bias_net", "STE", False), ("resnet18", "STE", False), ("rfdn", "LSQ", False)]
+          ("bias_net", "STE", False), ("asym_net", "STE", False), ("resnet18", "STE", False),
+          ("rfdn", "LSQ", False)]
 
 
 def _model(kind, method, channels_last):
@@ -174,12 +175,12 @@ def _ref64(codes_nchw, L, cw, stride, pad):
     """fp64 convolution of the exact dequantized values with the (folded) fp64 operands, and the
     bar terms |alpha S| + |beta SA| + |C| of the fp32 operands."""
     ca = codes_nchw.double()
-    c, k = cw.shape[1], cw.shape[2]
+    c, kh, kw = cw.shape[1:]
     a = ca * L.sa + L.zpa
     wt = cw.double() * L.sw.reshape(-1, 1, 1, 1) + L.zpw.reshape(-1, 1, 1, 1)
     ref = F.conv2d(a, wt, L.bias, stride=stride, padding=pad)
     s = F.conv2d(ca, cw.double(), stride=stride, padding=pad)
-    sam = F.conv2d(ca, torch.ones(1, c, k, k, dtype=torch.float64, device=DEV), stride=stride, padding=pad)
+    sam = F.conv2d(ca, torch.ones(1, c, kh, kw, dtype=torch.float64, device=DEV), stride=stride, padding=pad)
     hc, wc, nwc, ctab = L.pattern_tables(ca.shape[2], ca.shape[3], stride, pad)
     cterm = ctab.double()[hc.long()[:, None] * nwc + wc.long()[None, :]].permute(2, 0, 1)[None]
     terms = ((L.alpha.double().reshape(1, -1, 1, 1) * s).abs() + (L.beta.double().reshape(1, -1, 1, 1) * sam).abs()

@@ -272,6 +272,37 @@ class _BiasNet(nn.Module):
         return self.fc(torch.nn.functional.adaptive_avg_pool2d(x, 1).flatten(1))
 
 
+class _AsymNet(nn.Module):
+    """Classifier with per-axis convolution geometry: a (1, 3) stride-(1, 2) conv, a (3, 1) conv ->
+    BN -> ReLU, a residual block whose shortcut is a 1x1 stride-2 conv (which the quantizer leaves in
+    fp32, as ResNet-18's downsample), a 3x3 pad-2 conv on a 4 x 4 map (border outputs with a single
+    valid tap row) and a 1000-way Linear head.  Every quantized convolution carries a bias: with
+    quantize_bias the bias quantizer needs one (as in the reference's NoisyConv2d), and the BatchNorm
+    fold takes it into C."""
+
+    def __init__(self):
+        super().__init__()
+        self.c1 = nn.Conv2d(3, 16, (1, 3), stride=(1, 2), padding=(0, 1))
+        self.c2 = nn.Conv2d(16, 16, (3, 1), padding=(1, 0))
+        self.bn2 = nn.BatchNorm2d(16)
+        self.b1 = nn.Conv2d(16, 32, 3, stride=2, padding=1)
+        self.bn_b1 = nn.BatchNorm2d(32)
+        self.b2 = nn.Conv2d(32, 32, 3, padding=1)
+        self.bn_b2 = nn.BatchNorm2d(32)
+        self.downsample = nn.Sequential(nn.Conv2d(16, 32, 1, stride=2, bias=False), nn.BatchNorm2d(32))
+        self.c3 = nn.Conv2d(32, 32, 3, padding=2)
+        self.fc = nn.Linear(32, 1000)
+
+    def forward(self, x):
+        x = torch.relu(self.c1(x))                                   # 32 x 16
+        x = torch.relu(self.bn2(self.c2(x)))
+        y = torch.relu(self.bn_b1(self.b1(x)))                       # 16 x 8
+        x = torch.relu(self.bn_b2(self.b2(y)) + self.downsample(x))
+        x = torch.nn.functional.avg_pool2d(x, (4, 2))                # 4 x 4
+        x = torch.relu(self.c3(x))                                   # 6 x 6
+        return self.fc(torch.nn.functional.adaptive_avg_pool2d(x, 1).flatten(1))
+
+
 def _build(kind, method, channels_last=False, calib=True):
     torch.manual_seed(0)
     if kind == "resnet20":
@@ -281,7 +312,7 @@ def _build(kind, method, channels_last=False, calib=True):
         model, excl, qb = harness.build_model("resnet20"), harness.EXCLUDED["resnet20"], False
         qscheme = 0
     else:
-        model, excl, qb, qscheme = _BiasNet(), (), True, 1
+        model, excl, qb, qscheme = (_AsymNet() if kind == "asym_net" else _BiasNet()), (), True, 1
     lm = harness.LModule(model.to(DEV), nn.CrossEntropyLoss())
     cfg = harness.make_config(act_bit=4, weight_bit=4, qscheme=qscheme, qnmethod=method,
                               excluded_layers=excl, quantize_bias=qb)

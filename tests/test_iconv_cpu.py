@@ -27,28 +27,37 @@ from tests import pack_ref as R
 # ---------------------------------------------------------------------------------------------
 # the expansion of DESIGN §3 against fp64 convolution
 # ---------------------------------------------------------------------------------------------
-CASES = [  # (C, N, k, stride, pad, H, W)
-    (3, 8, 3, 1, 1, 9, 7),
-    (5, 4, 3, 2, 1, 10, 11),
-    (16, 6, 1, 1, 0, 5, 5),
-    (4, 3, 7, 2, 3, 12, 9),
-    (12, 5, 3, 2, 0, 9, 9),
-    (2, 3, 7, 1, 3, 5, 6),       # kernel wider than the image: every pixel is a border pixel
-    (6, 4, 1, 2, 0, 7, 8),
-    (7, 2, 3, 1, 0, 4, 4),
+CASES = [  # (C, N, (kh, kw), (sh, sw), (ph, pw), H, W)
+    (3, 8, (3, 3), (1, 1), (1, 1), 9, 7),
+    (5, 4, (3, 3), (2, 2), (1, 1), 10, 11),
+    (16, 6, (1, 1), (1, 1), (0, 0), 5, 5),
+    (4, 3, (7, 7), (2, 2), (3, 3), 12, 9),
+    (12, 5, (3, 3), (2, 2), (0, 0), 9, 9),
+    (2, 3, (7, 7), (1, 1), (3, 3), 5, 6),       # kernel wider than the image: every pixel is a border pixel
+    (6, 4, (1, 1), (2, 2), (0, 0), 7, 8),
+    (7, 2, (3, 3), (1, 1), (0, 0), 4, 4),
+    # per-axis geometry
+    (4, 5, (1, 3), (1, 2), (0, 1), 9, 12),
+    (3, 4, (3, 1), (1, 1), (1, 0), 10, 7),
+    (5, 3, (5, 3), (1, 3), (0, 0), 13, 14),
+    (6, 4, (7, 3), (2, 1), (3, 0), 15, 9),
+    (3, 5, (2, 4), (2, 1), (1, 2), 9, 10),
+    (4, 3, (2, 3), (3, 4), (1, 0), 12, 13),     # stride larger than the kernel
+    (3, 4, (3, 3), (1, 1), (3, 3), 2, 2),       # pad >= k: outputs with no valid tap
+    (5, 2, (3, 3), (1, 1), (4, 1), 1, 1),
+    (4, 3, (1, 1), (3, 2), (0, 0), 11, 10),
 ]
-
 
 @pytest.mark.parametrize("case", CASES)
 @pytest.mark.parametrize("zpa_nonzero", [False, True])
 @pytest.mark.parametrize("per_channel", [False, True])
 @pytest.mark.parametrize("with_bias", [False, True])
 def test_expansion_equals_fp64_conv(case, zpa_nonzero, per_channel, with_bias):
-    c, n, k, stride, pad, h, w = case
+    c, n, (kh, kw), stride, pad, h, w = case
     g = torch.Generator().manual_seed(hash((case, zpa_nonzero, per_channel, with_bias)) & 0xFFFF)
     a_top, w_top = 15, 7
     ca = torch.randint(0, a_top + 1, (2, c, h, w), generator=g)
-    cw = torch.randint(0, w_top + 1, (n, c, k, k), generator=g)
+    cw = torch.randint(0, w_top + 1, (n, c, kh, kw), generator=g)
     sa = 2.0 ** -5
     zpa = -1.375 if zpa_nonzero else 0.0
     rows = n if per_channel else 1
@@ -62,10 +71,14 @@ def test_expansion_equals_fp64_conv(case, zpa_nonzero, per_channel, with_bias):
     ref = F.conv2d(a, wt, None if bias is None else bias.double(), stride=stride, padding=pad)
 
     s = F.conv2d(ca.double(), cw.double(), stride=stride, padding=pad)
-    sa_m = F.conv2d(ca.double(), torch.ones(1, c, k, k, dtype=torch.float64), stride=stride, padding=pad)
-    hc, hv = ops.tap_classes(h, k, stride, pad)
-    wc, wv = ops.tap_classes(w, k, stride, pad)
+    sa_m = F.conv2d(ca.double(), torch.ones(1, c, kh, kw, dtype=torch.float64), stride=stride, padding=pad)
+    hc, hv = ops.tap_classes(h, kh, stride[0], pad[0])
+    wc, wv = ops.tap_classes(w, kw, stride[1], pad[1])
     ctab = L.constant_table(hv, wv)                               # fp64 [classes, N]
+    # the cached tables of the layer are the same classes
+    phc, pwc, nwc, pctab = L.pattern_tables(h, w, stride, pad)
+    assert torch.equal(phc, hc) and torch.equal(pwc, wc) and nwc == wv.shape[0]
+    assert torch.equal(pctab, ctab.float())
     p = hc.long()[:, None] * wv.shape[0] + wc.long()[None, :]     # [Ho, Wo]
     cterm = ctab[p].permute(2, 0, 1)[None]                        # [1, N, Ho, Wo]
     swn, zpwn = L.sw.reshape(1, -1, 1, 1), L.zpw.reshape(1, -1, 1, 1)
@@ -83,6 +96,30 @@ def test_tap_classes():
     assert valid[cls[0]].tolist() == [False, True, True] and valid[cls[7]].tolist() == [True, True, False]
     cls, valid = ops.tap_classes(1, 1, 1, 0)                      # a linear layer: one pattern
     assert cls.tolist() == [0] and valid.tolist() == [[True]]
+
+
+@pytest.mark.parametrize("size,k,stride,pad", [
+    (2, 3, 1, 3), (1, 3, 1, 4), (5, 1, 1, 1), (1, 1, 1, 2), (4, 2, 3, 2),          # pad >= k
+    (12, 2, 3, 1), (11, 1, 3, 0), (13, 3, 4, 0), (9, 1, 2, 0),                     # stride > k
+])
+def test_tap_classes_against_direct_enumeration(size, k, stride, pad):
+    """Each output position's class holds exactly its taps inside [0, size); with pad >= k some
+    position has no valid tap at all, with stride > k some input positions are never read."""
+    cls, valid = ops.tap_classes(size, k, stride, pad)
+    out = (size + 2 * pad - k) // stride + 1
+    assert cls.shape == (out,) and valid.shape[1] == k
+    assert len({tuple(v) for v in valid.tolist()}) == valid.shape[0]              # classes are distinct
+    for o in range(out):
+        want = [0 <= o * stride - pad + t < size for t in range(k)]
+        assert valid[cls[o]].tolist() == want, (o, want)
+    empty = [o for o in range(out) if not valid[cls[o]].any()]
+    if pad >= k:
+        assert empty == [o for o in range(out) if o * stride - pad + k <= 0 or o * stride - pad >= size] != []
+    else:
+        assert not empty
+    if stride > k:
+        read = {o * stride - pad + t for o in range(out) for t in range(k)}
+        assert set(range(size)) - read
 
 
 # ---------------------------------------------------------------------------------------------
@@ -270,8 +307,11 @@ def test_abi_argument_errors_without_gpu():
     assert iconv(h=1, ph=0) == -1                  # kernel larger than the padded image
     assert iconv(at=0) == -1 and iconv(wt=256) == -1
     assert iconv(codes=ctypes.c_void_p(24)) == -1  # not 16-byte aligned
-    # int32 bound: K * 255 * 255 >= 2^31 at K = 3*3*4096
+    # int32 bound: K * 255 * 255 >= 2^31 at K = 3*3*4096, and the first refused K of each kernel size
+    # (K = 33024 and 3 * 3 * 3664 are accepted: tests/test_gpu_iconv_limits.py runs them)
     assert iconv(cp=4096, at=255, wt=255) == -1
+    assert iconv(kh=1, kw=1, ph=0, pw=0, cp=33040, at=255, wt=255) == -1
+    assert iconv(cp=3680, at=255, wt=255) == -1
     # layout helper
     assert L.mhaq_fq_iconv_weight_bytes(0, 16, None, None, None, None) == -1
     assert L.mhaq_fq_iconv_weight_bytes(10, 24, None, None, None, None) == -1

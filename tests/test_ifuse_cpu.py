@@ -24,7 +24,7 @@ from mhaq_b200.quantization.gdnsq.inference import FusedIntegerConv2d, IntegerCo
 from mhaq_b200.quantization.gdnsq.layers.gdnsq_act import NoisyAct
 from mhaq_b200.quantization.gdnsq.layers.gdnsq_conv2d import NoisyConv2d
 from mhaq_b200.quantization.quantizer import Quantizer
-from tests.test_gpu_pack import _BiasNet
+from tests.test_gpu_pack import _AsymNet, _BiasNet
 from tests.test_iconv_cpu import CASES, _blob
 
 
@@ -48,11 +48,11 @@ def _bn(n, g, affine=True, tiny_var=False, negative=False):
 @pytest.mark.parametrize("bn_kind", ["plain", "negative_gamma", "tiny_var", "no_affine"])
 @pytest.mark.parametrize("per_channel,with_bias", [(True, True), (False, False), (True, False)])
 def test_batchnorm_fold_equals_fp64_batchnorm_of_fp64_conv(case, bn_kind, per_channel, with_bias):
-    c, n, k, stride, pad, h, w = case
+    c, n, (kh, kw), stride, pad, h, w = case
     g = torch.Generator().manual_seed(hash((case, bn_kind, per_channel, with_bias)) & 0xFFFF)
     a_top, w_top = 15, 7
     ca = torch.randint(0, a_top + 1, (2, c, h, w), generator=g)
-    cw = torch.randint(0, w_top + 1, (n, c, k, k), generator=g)
+    cw = torch.randint(0, w_top + 1, (n, c, kh, kw), generator=g)
     sa, zpa = 2.0 ** -5, -1.375
     rows = n if per_channel else 1
     sw = torch.exp2(torch.randint(-9, -5, (rows,), generator=g).float())
@@ -73,9 +73,9 @@ def test_batchnorm_fold_equals_fp64_batchnorm_of_fp64_conv(case, bn_kind, per_ch
            * gamma.reshape(1, -1, 1, 1) + beta.reshape(1, -1, 1, 1))
 
     s = F.conv2d(ca.double(), cw.double(), stride=stride, padding=pad)
-    sa_m = F.conv2d(ca.double(), torch.ones(1, c, k, k, dtype=torch.float64), stride=stride, padding=pad)
-    hc, hv = ops.tap_classes(h, k, stride, pad)
-    wc, wv = ops.tap_classes(w, k, stride, pad)
+    sa_m = F.conv2d(ca.double(), torch.ones(1, c, kh, kw, dtype=torch.float64), stride=stride, padding=pad)
+    hc, hv = ops.tap_classes(h, kh, stride[0], pad[0])
+    wc, wv = ops.tap_classes(w, kw, stride[1], pad[1])
     ctab = Lf.constant_table(hv, wv)
     p = hc.long()[:, None] * wv.shape[0] + wc.long()[None, :]
     cterm = ctab[p].permute(2, 0, 1)[None]
@@ -88,7 +88,7 @@ def test_batchnorm_fold_equals_fp64_batchnorm_of_fp64_conv(case, bn_kind, per_ch
     kk = gamma / torch.sqrt(var + bn.eps)
     assert torch.equal(Lf.sw, kk * L.sw) and torch.equal(Lf.zpw, kk * L.zpw)
     assert torch.equal(Lf.alpha, (sa * Lf.sw).float()) and torch.equal(Lf.beta, (sa * Lf.zpw).float())
-    assert torch.equal(Lf.pattern_tables(h, w, (stride, stride), (pad, pad))[3], ctab.float())
+    assert torch.equal(Lf.pattern_tables(h, w, stride, pad)[3], ctab.float())
     # the weight operand is shared, the unfolded operands are untouched
     assert Lf.weight is L.weight and torch.equal(L.alpha, (sa * L.sw).float())
 
@@ -110,8 +110,8 @@ def _integer_stand_in(name):
     """build_integer_model of the quantized harness model (or the biased test net) with a
     synthetic export: the structure is what the pass sees, the numbers do not matter here."""
     torch.manual_seed(0)
-    if name == "bias_net":      # per tensor: the synthetic export has per-tensor Linear weights
-        model, excl, qb, qscheme = _BiasNet(), (), False, 0
+    if name in ("bias_net", "asym_net"):   # per tensor: the synthetic export has per-tensor Linear weights
+        model, excl, qb, qscheme = (_BiasNet() if name == "bias_net" else _AsymNet()), (), False, 0
     else:
         model, excl, qb, qscheme = harness.build_model(name), harness.EXCLUDED[name], False, 1
     lm = (harness.SRModule if name == "rfdn" else harness.LModule)(model, nn.MSELoss())
@@ -148,6 +148,10 @@ STRUCTURE = {
     "rfdn": ({"codes": 12, "fp32": 9, "both": 8}, 13, 4),
     # c1 -> relu -> c2 (codes), c2 -> relu -> pool (fp32, codes in); the Linear head keeps act_codes
     "bias_net": ({"codes": 1, "fp32": 1}, 2, 0),
+    # c1 (1x3) -> relu -> c2 (codes); c2 (3x1) -> bn -> relu feeds b1 and the fp32 downsample
+    # (both); b1 -> bn -> relu -> b2 (codes); b2 -> bn -> + downsample -> relu -> pool and
+    # c3 -> relu -> pool (fp32).  c1, c3 and the Linear head quantize fp32: 3 act_codes inputs
+    "asym_net": ({"codes": 2, "both": 1, "fp32": 2}, 3, 0),
 }
 
 
