@@ -41,6 +41,9 @@
  *   mhaq_fq_iconv_fused_u8     mhaq_fq_iconv_u8 with an eval BatchNorm folded into its operands and
  *                              the residual add, ReLU / LeakyReLU and the next layer's codes in its
  *                              epilogue
+ *   mhaq_fq_iconv_grouped_u8   a grouped, depthwise or dilated integer convolution with the fused
+ *                              epilogue: depthwise on the CUDA cores, the rest on the tensor cores
+ *   mhaq_fq_iconv_grouped_weight_bytes  the size and tiling of its weight operand
  *   mhaq_fq_potential_loss_*   PotentialLoss.forward's constraint arithmetic and its autograd
  *                              (gdnsq_loss.py:32-86, 114-168), one launch each way
  *
@@ -460,6 +463,53 @@ int mhaq_fq_iconv_fused_u8(const uint8_t *codes, const uint8_t *weights, const f
                            int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                            int act_max_code, int weight_max_code, const mhaq_fq_iconv_epilogue *epilogue,
                            void *stream);
+
+/* Grouped and dilated integer convolutions (DESIGN.md §3 "Grouped and dilated layers").
+ *   The layer has n_in input and n_out output channels in `groups` groups (both divisible by it);
+ *   output channel n of group g(n) = n / (n_out / groups) sums over the cin_g = n_in / groups input
+ *   channels of its group and the valid taps, tap (i, j) reading input position
+ *   (o_h * stride_h - pad_h + i * dilation_h, o_w * stride_w - pad_w + j * dilation_w).  The output is
+ *   ((height + 2 pad_h - dilation_h (kernel_h - 1) - 1) / stride_h + 1) x (... w ...).  The epilogue
+ *   is that of mhaq_fq_iconv_u8 with SA[m][g(n)] the sum of the group's codes and |p| counting
+ *   valid taps x cin_g.
+ *
+ * mhaq_fq_iconv_grouped_weight_bytes: bytes of the weight operand; -1 for a bad geometry.
+ *   Depthwise (groups == n_in == n_out): u8 [kernel_h * kernel_w][cp], cp = round_up(n_in, 16),
+ *   padding channels 0; *n_tiles = *tile_n = *tile_out = *groups_per_tile = *tiles_per_group =
+ *   *k_stages = 0.  Otherwise N tiles as in mhaq_fq_iconv_weight_bytes, block-diagonal: when a group
+ *   with its ones row fits a tile, tile t holds groups_per_tile whole groups
+ *   [t * groups_per_tile, ...) (tiles_per_group = 1), their tile_out = groups_per_tile * cout_g
+ *   channels, then one ones row per group (row tile_out + i for the tile's i-th group); otherwise
+ *   each group spans tiles_per_group tiles of at most tile_out channels and one ones row
+ *   (groups_per_tile = 1).  Tile t's K is (kh, kw, chunks [c_lo, c_hi)) with
+ *   c_lo = floor(first group * cin_g / 16), c_hi = ceil(end group * cin_g / 16): a row holds its
+ *   channel's weights at its own group's channels and 0 elsewhere, a ones row is 1 exactly at its
+ *   group's channels.  Each row is zero-padded to k_stages * 128 bytes (the widest tile's K) and
+ *   stored like mhaq_fq_iconv_weight_bytes' operand.  Any output pointer may be NULL.
+ *
+ * mhaq_fq_iconv_grouped_u8: codes [batch][height][width][cp] (16-byte aligned), the weight operand
+ *   above (16-byte aligned), alpha / beta [n_out], ctab [n_h_classes * n_w_classes][n_out] and
+ *   h_class / w_class of the dilated tap patterns; the outputs as in mhaq_fq_iconv_fused_u8 (an
+ *   epilogue with y alone is the plain layer).  Depthwise layers run on the CUDA cores, all others
+ *   on the tensor cores.  Errors (before any CUDA call): those of mhaq_fq_iconv_fused_u8, groups
+ *   that do not divide n_in and n_out, a dilation below 1, and
+ *   kernel_h * kernel_w * cin_g * act_max_code * weight_max_code >= 2^31.  Capture-safe. */
+typedef struct mhaq_fq_iconv_geometry {
+    int kernel_h, kernel_w;
+    int stride_h, stride_w;
+    int pad_h, pad_w;
+    int dilation_h, dilation_w;
+    int groups;
+} mhaq_fq_iconv_geometry;
+
+int64_t mhaq_fq_iconv_grouped_weight_bytes(int64_t n_in, int64_t n_out, const mhaq_fq_iconv_geometry *geometry,
+                                           int *n_tiles, int *tile_n, int *tile_out, int *groups_per_tile,
+                                           int *tiles_per_group, int64_t *k_stages);
+int mhaq_fq_iconv_grouped_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                             const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                             int64_t batch, int64_t height, int64_t width, int64_t n_in, int64_t n_out,
+                             const mhaq_fq_iconv_geometry *geometry, int act_max_code, int weight_max_code,
+                             const mhaq_fq_iconv_epilogue *epilogue, void *stream);
 
 #ifdef __cplusplus
 }

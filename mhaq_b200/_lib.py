@@ -39,6 +39,12 @@ class IConvEpilogue(ctypes.Structure):
 
 ACT_NONE, ACT_RELU, ACT_LEAKY_RELU = 0, 1, 2  # MHAQ_FQ_ACT_*
 
+
+class IConvGeometry(ctypes.Structure):
+    """mhaq_fq_iconv_geometry"""
+    _fields_ = [(n, c_int) for n in ("kernel_h", "kernel_w", "stride_h", "stride_w", "pad_h", "pad_w",
+                                     "dilation_h", "dilation_w", "groups")]
+
 # name -> (restype, argtypes); mirrors include/mhaq_fq.h one to one
 _P = c_void_p
 _SIGNATURES = {
@@ -89,6 +95,9 @@ _SIGNATURES = {
                                  c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P]),
     "mhaq_fq_iconv_fused_u8": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int64, c_int64, c_int64, c_int64,
                                        c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "mhaq_fq_iconv_grouped_weight_bytes": (c_int64, [c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P]),
+    "mhaq_fq_iconv_grouped_u8": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int64, c_int64, c_int64, c_int64,
+                                         c_int64, _P, c_int, c_int, _P, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

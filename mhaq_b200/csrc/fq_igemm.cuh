@@ -60,6 +60,73 @@ __host__ __device__ inline IcLayout iconv_layout(int64_t n_out, int64_t k_bytes)
     return l;
 }
 
+// N tiling of a grouped (or dilated, one-group) weight operand: a pure function of (n_out, groups,
+// cin_g, kh, kw).  When a group and its ones row fit one tile (cout_g + 1 <= 256), a tile holds gpt
+// whole groups: tile_out = gpt * cout_g output channels, then gpt ones rows (local row tile_out + i
+// for the tile's i-th group), tile_out + gpt <= 256 rounded up to 16.  Otherwise every group spans
+// `parts` tiles of at most 255 channels and one ones row, one group per tile (gpt = 1).  A tile's K
+// is (kh, kw, its groups' input channels rounded out to 16-channel chunks), so the tiles' K widths
+// differ; every tile runs the widest tile's k_stages with the rest zero-filled.
+struct IgPlan {
+    int n_tiles, tile_n, tile_out, gpt, parts;
+    int64_t k_stages;
+};
+// Output channels [n_base, n_base + n_here), groups [g_lo, g_lo + n_grp) and 16-channel input chunks
+// [c_lo, c_lo + kc) of one tile.
+struct IgTile {
+    int64_t n_base, n_here, g_lo, c_lo, kc;
+    int n_grp;
+};
+__host__ __device__ inline IgTile igroup_tile(int64_t groups, int64_t cin_g, int64_t cout_g, int tile_out, int gpt,
+                                              int parts, int tile) {
+    IgTile t;
+    int64_t g_hi, n_end;
+    if (parts == 1) {
+        t.g_lo = (int64_t)tile * gpt;
+        g_hi = t.g_lo + gpt < groups ? t.g_lo + gpt : groups;
+        t.n_base = t.g_lo * cout_g;
+        n_end = g_hi * cout_g;
+    } else {
+        t.g_lo = tile / parts;
+        g_hi = t.g_lo + 1;
+        t.n_base = t.g_lo * cout_g + (int64_t)(tile % parts) * tile_out;
+        n_end = t.n_base + tile_out < g_hi * cout_g ? t.n_base + tile_out : g_hi * cout_g;
+    }
+    t.n_here = n_end - t.n_base;
+    t.n_grp = (int)(g_hi - t.g_lo);
+    t.c_lo = t.g_lo * cin_g / 16;
+    t.kc = (g_hi * cin_g + 15) / 16 - t.c_lo;
+    return t;
+}
+inline IgPlan igroup_plan(int64_t n_out, int64_t groups, int64_t cin_g, int kh, int kw) {
+    IgPlan l;
+    const int64_t cout_g = n_out / groups;
+    if (cout_g + 1 <= kIcMaxTileN) {
+        // as many whole groups as fit, then as few tiles of that many groups as cover them all
+        int64_t gpt = kIcMaxTileN / (cout_g + 1);
+        if (gpt > groups) gpt = groups;
+        const int64_t nt = (groups + gpt - 1) / gpt;
+        l.gpt = (int)((groups + nt - 1) / nt);
+        l.n_tiles = (int)((groups + l.gpt - 1) / l.gpt);
+        l.parts = 1;
+        l.tile_out = (int)(l.gpt * cout_g);
+    } else {
+        const int64_t p_min = (cout_g + kIcMaxTileN - 2) / (kIcMaxTileN - 1);
+        l.tile_out = (int)((cout_g + p_min - 1) / p_min);
+        l.parts = (int)((cout_g + l.tile_out - 1) / l.tile_out);
+        l.gpt = 1;
+        l.n_tiles = (int)(groups * l.parts);
+    }
+    l.tile_n = (l.tile_out + l.gpt + 15) / 16 * 16;
+    int64_t kc_max = 0;
+    for (int t = 0; t < l.n_tiles; ++t) {
+        const IgTile g = igroup_tile(groups, cin_g, cout_g, l.tile_out, l.gpt, l.parts, t);
+        if (g.kc > kc_max) kc_max = g.kc;
+    }
+    l.k_stages = ((int64_t)kh * kw * kc_max + 7) / 8;
+    return l;
+}
+
 // ---------------------------------------------------------------------------------------------
 // activation codes
 // ---------------------------------------------------------------------------------------------
@@ -183,6 +250,10 @@ struct IConvArgs {
     float slope;               // LeakyReLU negative slope
     int act;                   // kIcAct*
     int vec_res;               // res 16-byte aligned and n_out % 4 == 0: float4 loads
+    // grouped / dilated layers (fq_iconv_kernel<true, true>, fq_idw_kernel)
+    int dh, dw;                // dilation
+    int64_t groups, cin_g, cout_g;
+    int gpt, parts;            // IgPlan
 };
 
 constexpr int kIcActNone = 0, kIcActRelu = 1, kIcActLeaky = 2;   // = MHAQ_FQ_ACT_*
@@ -267,7 +338,11 @@ __device__ __forceinline__ void iconv_fused_chunk(const IConvArgs &p, float (&ou
 // FUSED = false: y = alpha * S + beta * SA + C, fp32 only (mhaq_fq_iconv_u8).  FUSED = true: the
 // same value through iconv_fused_chunk (mhaq_fq_iconv_fused_u8); the tile holding the last output
 // channels also writes the codes' padding channels [n_out, cp_out) as 0.
-template <bool FUSED>
+// GROUPED = true (with FUSED, mhaq_fq_iconv_grouped_u8): block-diagonal N tiles of IgPlan.  The
+// producers gather only the tile's input chunks [c_lo, c_lo + kc) of each tap, at dilated tap
+// offsets; the epilogue reads channel n's SA from the ones column of its group, which it first
+// copies from tensor memory into the (then idle) A stages, [group][row].
+template <bool FUSED, bool GROUPED = false>
 __global__ void __launch_bounds__(kIcThreads, 1)
 fq_iconv_kernel(const IConvArgs p) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -319,7 +394,10 @@ fq_iconv_kernel(const IConvArgs p) {
             wi0[i] = ow * p.sw - p.pw;
             row_base[i] = p.a + img * p.h * p.w * p.cp;
         }
-        const int64_t cpc = p.cp / 16;        // 16-byte chunks per tap
+        [[maybe_unused]] IgTile gt{};
+        if constexpr (GROUPED) gt = igroup_tile(p.groups, p.cin_g, p.cout_g, p.tile_out, p.gpt, p.parts, tile);
+        const int64_t cpc = GROUPED ? gt.kc : p.cp / 16;        // 16-byte chunks per tap
+        [[maybe_unused]] const int64_t g_chunks = GROUPED ? (int64_t)p.kh * p.kw * gt.kc : 0;
         const uint8_t *bsrc = p.b + (int64_t)tile * p.k_stages * b_stage;
         for (int64_t kt = 0; kt < p.k_stages; ++kt) {
             const int s = (int)(kt % kIcStages);
@@ -329,13 +407,14 @@ fq_iconv_kernel(const IConvArgs p) {
             for (int j = 0; j < 4; ++j) {
                 const int c = 2 * j + sub;
                 const int64_t q = kt * 8 + c;               // global 16-byte chunk of K
-                const int64_t tap = q / cpc, cc = q - tap * cpc;
+                const int64_t tap = q / cpc, cc = q - tap * cpc + (GROUPED ? gt.c_lo : 0);
                 const int64_t tkh = tap / p.kw, tkw = tap - tkh * p.kw;
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
                     const int r = rr + 64 * i;
-                    const int64_t ih = hi0[i] + tkh, iw = wi0[i] + tkw;
-                    const bool ok = row_ok[i] && q < p.k_chunks && ih >= 0 && ih < p.h && iw >= 0 && iw < p.w;
+                    const int64_t ih = hi0[i] + (GROUPED ? tkh * p.dh : tkh), iw = wi0[i] + (GROUPED ? tkw * p.dw : tkw);
+                    const bool ok = row_ok[i] && q < (GROUPED ? g_chunks : p.k_chunks) && ih >= 0 && ih < p.h &&
+                                    iw >= 0 && iw < p.w;
                     const uint8_t *src = ok ? row_base[i] + ((ih * p.w + iw) * p.cp + cc * 16) : p.a;
                     cp_async16(a_dst + (r >> 3) * 1024 + c * 128 + (r & 7) * 16, src, ok ? 16 : 0);
                 }
@@ -358,9 +437,27 @@ fq_iconv_kernel(const IConvArgs p) {
         mbar_wait(accum, 0);
         tc_fence_after();
         const uint32_t lane_addr = tmem + ((uint32_t)(warp * 32) << 16);
-        uint32_t sa_u;
-        tmem_ld1(lane_addr + p.tile_out, sa_u);
-        tmem_wait_ld();
+        [[maybe_unused]] uint32_t sa_u;
+        [[maybe_unused]] uint32_t *sas = reinterpret_cast<uint32_t *>(sa);
+        if constexpr (GROUPED) {
+            // the ones columns tile_out + [0, n_grp) -> sas[group][row]; the MMAs that read the A
+            // stages are complete (accum), so the stages are free.  A 16-column load starts at most
+            // at tile_n - 16 so that it stays inside the tile's columns.
+            for (int g0 = 0; g0 < gt.n_grp; g0 += 16) {
+                const int base = p.tile_out + g0 < p.tile_n - 16 ? p.tile_out + g0 : p.tile_n - 16;
+                uint32_t v[16];
+                tmem_ld16(lane_addr + base, v);
+                tmem_wait_ld();
+#pragma unroll
+                for (int i = 0; i < 16; ++i) {
+                    const int g = base - p.tile_out + i;
+                    if (g >= g0 && g < gt.n_grp) sas[g * kIcTileM + tid] = v[i];
+                }
+            }
+        } else {
+            tmem_ld1(lane_addr + p.tile_out, sa_u);
+            tmem_wait_ld();
+        }
         const int64_t m = m0 + tid;                  // TMEM lane tid = row tid of the tile
         const bool live = m < p.m;
         int64_t ctab_row = 0;
@@ -369,9 +466,10 @@ fq_iconv_kernel(const IConvArgs p) {
             const int64_t oh = rem / p.wo, ow = rem - oh * p.wo;
             ctab_row = ((int64_t)__ldg(p.hcls + oh) * p.n_wcls + __ldg(p.wcls + ow)) * p.n_out;
         }
-        const double sa_d = (double)sa_u;
-        const int64_t n_base = (int64_t)tile * p.tile_out;
-        const int64_t n_here = (p.n_out - n_base) < p.tile_out ? (p.n_out - n_base) : p.tile_out;
+        [[maybe_unused]] const double sa_d = GROUPED ? 0.0 : (double)sa_u;
+        const int64_t n_base = GROUPED ? gt.n_base : (int64_t)tile * p.tile_out;
+        const int64_t n_here =
+            GROUPED ? gt.n_here : ((p.n_out - n_base) < p.tile_out ? (p.n_out - n_base) : p.tile_out);
         float *yrow = p.y + m * p.n_out + n_base;
         const bool vec = p.vec_out && (n_base & 3) == 0;
         QConst cq{};
@@ -398,15 +496,27 @@ fq_iconv_kernel(const IConvArgs p) {
             tmem_wait_ld();
             if (!live) continue;
             float out[16];
+            [[maybe_unused]] int64_t gq = 0, gr = 0;     // the column's group within the tile, and its rank in it
+            if constexpr (GROUPED) {
+                gq = col / p.cout_g;
+                gr = col - gq * p.cout_g;
+            }
 #pragma unroll
             for (int i = 0; i < 16; ++i) {
                 const int64_t n = n_base + col + i;
                 if (col + i < n_here) {
                     // fp64: alpha * S and beta * SA carry at most one rounding each, the result one
-                    const double t = __fma_rn((double)__ldg(p.beta + n), sa_d, (double)__ldg(p.ctab + ctab_row + n));
+                    const double sa_n = GROUPED ? (double)sas[gq * kIcTileM + tid] : sa_d;
+                    const double t = __fma_rn((double)__ldg(p.beta + n), sa_n, (double)__ldg(p.ctab + ctab_row + n));
                     out[i] = __double2float_rn(__fma_rn((double)__ldg(p.alpha + n), (double)(int32_t)v[i], t));
                 } else {
                     out[i] = 0.f;
+                }
+                if constexpr (GROUPED) {
+                    if (++gr == p.cout_g) {
+                        gr = 0;
+                        ++gq;
+                    }
                 }
             }
             if constexpr (FUSED) {
@@ -453,4 +563,88 @@ fq_iconv_kernel(const IConvArgs p) {
 
 inline size_t iconv_smem_bytes(int tile_n) {
     return (size_t)kIcStages * (kIcAStage + tile_n * kIcStageK) + (2 * kIcStages + 1) * 8 + 16;
+}
+
+// ---------------------------------------------------------------------------------------------
+// depthwise convolution on the CUDA cores (groups == cin == n_out)
+// ---------------------------------------------------------------------------------------------
+// One channel's sum has only kh * kw terms, so block-diagonal MMA tiles would multiply zeros almost
+// everywhere.  Instead one thread per (output pixel, 16-channel chunk) loads one 16-byte code
+// vector and one 16-byte weight vector per valid tap and accumulates S and SA of its 16 channels
+// in int32; the weight operand is u8 [kh * kw][cp].  Consecutive threads take consecutive chunks
+// of one pixel, so a warp's code loads are contiguous.  The epilogue is fq_iconv_kernel<true>'s:
+// the same fp64 sum, then iconv_fused_chunk.  Grid-stride, 64-bit offsets; no host
+// synchronisation, allocation or atomic.
+constexpr int kDwThreads = 256;
+
+__device__ __forceinline__ void dw_acc4(uint32_t a, uint32_t w, int32_t *s, int32_t *sa) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int32_t av = (int32_t)((a >> (8 * j)) & 0xffu), wv = (int32_t)((w >> (8 * j)) & 0xffu);
+        s[j] += av * wv;
+        sa[j] += av;
+    }
+}
+
+__global__ void __launch_bounds__(kDwThreads)
+fq_idw_kernel(const IConvArgs p) {
+    const int64_t cpc = p.cp / 16;
+    const int64_t total = p.m * cpc;
+    QConst cq{};
+    Div2 cdv{};
+    f32x2 czpn{}, czp2{};
+    bool cfast = false;
+    if (p.codes) {
+        const QParams prm = {p.code_s, p.code_zp, p.code_zp, p.code_hi, 0, 0, 0, 0, PARAMS_LINEAR};
+        cq = load_qconst(prm, 0);
+        cdv = make_div2(cq.s, __frcp_rn(cq.s));
+        czpn = bc2(-cq.zp);
+        czp2 = bc2(cq.zp);
+        cfast = scale_fast_ok(cq.s);
+    }
+    for (int64_t t = (int64_t)blockIdx.x * kDwThreads + threadIdx.x; t < total;
+         t += (int64_t)gridDim.x * kDwThreads) {
+        const int64_t m = t / cpc, ck = t - m * cpc;
+        const int64_t img = m / (p.ho * p.wo), rem = m - img * (p.ho * p.wo);
+        const int64_t oh = rem / p.wo, ow = rem - oh * p.wo;
+        const int64_t hi0 = oh * p.sh - p.ph, wi0 = ow * p.sw - p.pw;
+        const uint8_t *abase = p.a + img * p.h * p.w * p.cp + ck * 16;
+        const uint8_t *wbase = p.b + ck * 16;
+        int32_t s[16], sa[16];
+#pragma unroll
+        for (int i = 0; i < 16; ++i) s[i] = sa[i] = 0;
+        for (int th = 0; th < p.kh; ++th) {
+            const int64_t ih = hi0 + (int64_t)th * p.dh;
+            if (ih < 0 || ih >= p.h) continue;
+            for (int tw = 0; tw < p.kw; ++tw) {
+                const int64_t iw = wi0 + (int64_t)tw * p.dw;
+                if (iw < 0 || iw >= p.w) continue;
+                const uint4 av = __ldg(reinterpret_cast<const uint4 *>(abase + (ih * p.w + iw) * p.cp));
+                const uint4 wv = __ldg(reinterpret_cast<const uint4 *>(wbase + (int64_t)(th * p.kw + tw) * p.cp));
+                dw_acc4(av.x, wv.x, s, sa);
+                dw_acc4(av.y, wv.y, s + 4, sa + 4);
+                dw_acc4(av.z, wv.z, s + 8, sa + 8);
+                dw_acc4(av.w, wv.w, s + 12, sa + 12);
+            }
+        }
+        const int64_t n0 = ck * 16;
+        const int nv = p.n_out - n0 < 16 ? (int)(p.n_out - n0) : 16;
+        float rv[16];
+        if (p.res) iconv_load_res(p, rv, m, n0, nv);
+        const int64_t ctab_row = ((int64_t)__ldg(p.hcls + oh) * p.n_wcls + __ldg(p.wcls + ow)) * p.n_out;
+        float out[16];
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+            const int64_t n = n0 + i;
+            if (i < nv) {
+                const double u = __fma_rn((double)__ldg(p.beta + n), (double)sa[i], (double)__ldg(p.ctab + ctab_row + n));
+                out[i] = __double2float_rn(__fma_rn((double)__ldg(p.alpha + n), (double)s[i], u));
+            } else {
+                out[i] = 0.f;
+            }
+        }
+        iconv_fused_chunk(p, out, rv, m, n0, nv, p.vec_out, cq, cdv, czpn, czp2, cfast);
+        if (p.codes)
+            for (int i = nv; i < 16; ++i) p.codes[m * p.cp_out + n0 + i] = 0;
+    }
 }

@@ -1789,14 +1789,14 @@ void launch_unpack(bool vec, int grid, cudaStream_t st, const uint8_t *packed, f
 // ---- integer layers (fq_igemm.cuh) ----
 // The iconv kernel needs more than 48 KiB of dynamic shared memory: opt in once per device and
 // instantiation.
-template <bool FUSED>
+template <bool FUSED, bool GROUPED = false>
 inline int iconv_smem_opt_in() {
     static bool done[64] = {};
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return (int)e;
     if (dev < 64 && done[dev]) return 0;
-    e = cudaFuncSetAttribute(fq_iconv_kernel<FUSED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    e = cudaFuncSetAttribute(fq_iconv_kernel<FUSED, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)iconv_smem_bytes(kIcMaxTileN));
     if (e != cudaSuccess) return (int)e;
     if (dev < 64) done[dev] = true;
@@ -1840,6 +1840,90 @@ inline int iconv_args(const uint8_t *codes, const uint8_t *weights, const float 
     a.tmem_cols = 32;
     while (a.tmem_cols < l.tile_n) a.tmem_cols <<= 1;
     grid = dim3((unsigned)m_tiles, (unsigned)l.n_tiles);
+    return 0;
+}
+
+// Checks of a fused epilogue (no CUDA call).
+inline int iconv_epilogue_check(const mhaq_fq_iconv_epilogue *epilogue) {
+    if (!epilogue) return MHAQ_FQ_ENULL;
+    const mhaq_fq_iconv_epilogue &e = *epilogue;
+    if (!e.y && !e.codes) return MHAQ_FQ_EINVAL;
+    if (e.codes && (!e.code_scale || !e.code_zero_point || !e.code_max_val)) return MHAQ_FQ_ENULL;
+    if (e.codes && !aligned16(e.codes)) return MHAQ_FQ_EINVAL;
+    if (e.activation != MHAQ_FQ_ACT_NONE && e.activation != MHAQ_FQ_ACT_RELU &&
+        e.activation != MHAQ_FQ_ACT_LEAKY_RELU)
+        return MHAQ_FQ_EINVAL;
+    return 0;
+}
+
+// The epilogue's fields of `a` (after iconv_epilogue_check; a.n_out is set).
+inline void iconv_epilogue_set(const mhaq_fq_iconv_epilogue &e, IConvArgs &a) {
+    a.y = e.y;
+    a.vec_out = e.y && aligned16(e.y) && a.n_out % 4 == 0;
+    a.res = e.residual;
+    a.vec_res = e.residual && aligned16(e.residual) && a.n_out % 4 == 0;
+    a.act = e.activation;
+    a.slope = e.negative_slope;
+    a.codes = e.codes;
+    a.code_s = e.code_scale; a.code_zp = e.code_zero_point; a.code_hi = e.code_max_val;
+    a.cp_out = (a.n_out + 15) / 16 * 16;
+}
+
+inline bool igroup_depthwise(int64_t n_in, int64_t n_out, int groups) { return groups == n_in && groups == n_out; }
+
+// Geometry checks of a grouped / dilated layer (no CUDA call).
+inline int igroup_geometry_ok(int64_t n_in, int64_t n_out, const mhaq_fq_iconv_geometry &g) {
+    if (n_in < 1 || n_out < 1 || g.groups < 1 || n_in % g.groups != 0 || n_out % g.groups != 0) return 0;
+    if (g.kernel_h < 1 || g.kernel_w < 1 || g.stride_h < 1 || g.stride_w < 1 || g.pad_h < 0 || g.pad_w < 0)
+        return 0;
+    return g.dilation_h >= 1 && g.dilation_w >= 1;
+}
+
+// Argument checks and kernel arguments of mhaq_fq_iconv_grouped_u8 (no CUDA call).
+inline int igroup_args(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                       const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                       int64_t batch, int64_t height, int64_t width, int64_t n_in, int64_t n_out,
+                       const mhaq_fq_iconv_geometry *geometry, int act_max_code, int weight_max_code,
+                       const mhaq_fq_iconv_epilogue *epilogue, IConvArgs &a, IgPlan &l) {
+    const int rc = iconv_epilogue_check(epilogue);
+    if (rc) return rc;
+    if (!codes || !weights || !alpha || !beta || !ctab || !h_class || !w_class || !geometry) return MHAQ_FQ_ENULL;
+    const mhaq_fq_iconv_geometry g = *geometry;
+    if (!igroup_geometry_ok(n_in, n_out, g)) return MHAQ_FQ_EINVAL;
+    if (batch < 1 || height < 1 || width < 1 || n_w_classes < 1) return MHAQ_FQ_EINVAL;
+    if (act_max_code < 1 || act_max_code > 255 || weight_max_code < 1 || weight_max_code > 255)
+        return MHAQ_FQ_EINVAL;
+    if (!aligned16(codes) || !aligned16(weights)) return MHAQ_FQ_EINVAL;
+    // extent of the dilated kernel
+    const int64_t eh = (int64_t)g.dilation_h * (g.kernel_h - 1) + 1, ew = (int64_t)g.dilation_w * (g.kernel_w - 1) + 1;
+    if (height + 2 * g.pad_h < eh || width + 2 * g.pad_w < ew) return MHAQ_FQ_EINVAL;
+    const int64_t ho = (height + 2 * g.pad_h - eh) / g.stride_h + 1;
+    const int64_t wo = (width + 2 * g.pad_w - ew) / g.stride_w + 1;
+    const int64_t cin_g = n_in / g.groups;
+    // one channel's int32 sums: kh * kw * cin_g products, each at most act_max_code * weight_max_code
+    const int64_t terms = (int64_t)g.kernel_h * g.kernel_w * cin_g;
+    if (terms > (int64_t)1 << 31 || terms * act_max_code * weight_max_code >= ((int64_t)1 << 31))
+        return MHAQ_FQ_EINVAL;
+    a = IConvArgs{};
+    const int64_t m = batch * ho * wo;
+    const int64_t cp = (n_in + 15) / 16 * 16;
+    if (igroup_depthwise(n_in, n_out, g.groups)) {
+        l = IgPlan{};
+    } else {
+        l = igroup_plan(n_out, g.groups, cin_g, g.kernel_h, g.kernel_w);
+        if ((m + kIcTileM - 1) / kIcTileM > 0x7fffffffLL || l.n_tiles > 65535) return MHAQ_FQ_EINVAL;
+    }
+    a.a = codes; a.b = weights; a.alpha = alpha; a.beta = beta; a.ctab = ctab;
+    a.hcls = h_class; a.wcls = w_class;
+    a.m = m; a.h = height; a.w = width; a.cp = cp; a.n_out = n_out; a.ho = ho; a.wo = wo;
+    a.k_stages = l.k_stages;
+    a.kh = g.kernel_h; a.kw = g.kernel_w; a.sh = g.stride_h; a.sw = g.stride_w; a.ph = g.pad_h; a.pw = g.pad_w;
+    a.dh = g.dilation_h; a.dw = g.dilation_w;
+    a.groups = g.groups; a.cin_g = cin_g; a.cout_g = n_out / g.groups;
+    a.n_wcls = n_w_classes; a.tile_n = l.tile_n; a.tile_out = l.tile_out; a.gpt = l.gpt; a.parts = l.parts;
+    a.tmem_cols = 32;
+    while (a.tmem_cols < l.tile_n) a.tmem_cols <<= 1;
+    iconv_epilogue_set(*epilogue, a);
     return 0;
 }
 
@@ -2416,32 +2500,62 @@ int mhaq_fq_iconv_fused_u8(const uint8_t *codes, const uint8_t *weights, const f
                            int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                            int act_max_code, int weight_max_code, const mhaq_fq_iconv_epilogue *epilogue,
                            void *stream) {
-    if (!epilogue) return MHAQ_FQ_ENULL;
-    const mhaq_fq_iconv_epilogue &e = *epilogue;
-    if (!e.y && !e.codes) return MHAQ_FQ_EINVAL;
-    if (e.codes && (!e.code_scale || !e.code_zero_point || !e.code_max_val)) return MHAQ_FQ_ENULL;
-    if (e.codes && !aligned16(e.codes)) return MHAQ_FQ_EINVAL;
-    if (e.activation != MHAQ_FQ_ACT_NONE && e.activation != MHAQ_FQ_ACT_RELU &&
-        e.activation != MHAQ_FQ_ACT_LEAKY_RELU)
-        return MHAQ_FQ_EINVAL;
+    int rc = iconv_epilogue_check(epilogue);
+    if (rc) return rc;
     IConvArgs a;
     dim3 grid;
-    int rc = iconv_args(codes, weights, alpha, beta, ctab, h_class, w_class, n_w_classes, batch, height, width, cp,
-                        n_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, act_max_code, weight_max_code,
-                        a, grid);
+    rc = iconv_args(codes, weights, alpha, beta, ctab, h_class, w_class, n_w_classes, batch, height, width, cp,
+                    n_out, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, act_max_code, weight_max_code,
+                    a, grid);
     if (rc) return rc;
     rc = iconv_smem_opt_in<true>();
     if (rc) return rc;
-    a.y = e.y;
-    a.vec_out = e.y && aligned16(e.y) && n_out % 4 == 0;
-    a.res = e.residual;
-    a.vec_res = e.residual && aligned16(e.residual) && n_out % 4 == 0;
-    a.act = e.activation;
-    a.slope = e.negative_slope;
-    a.codes = e.codes;
-    a.code_s = e.code_scale; a.code_zp = e.code_zero_point; a.code_hi = e.code_max_val;
-    a.cp_out = (n_out + 15) / 16 * 16;
+    iconv_epilogue_set(*epilogue, a);
     fq_iconv_kernel<true><<<grid, kIcThreads, iconv_smem_bytes(a.tile_n), (cudaStream_t)stream>>>(a);
+    return last_error();
+}
+
+int64_t mhaq_fq_iconv_grouped_weight_bytes(int64_t n_in, int64_t n_out, const mhaq_fq_iconv_geometry *geometry,
+                                           int *n_tiles, int *tile_n, int *tile_out, int *groups_per_tile,
+                                           int *tiles_per_group, int64_t *k_stages) {
+    if (!geometry || !igroup_geometry_ok(n_in, n_out, *geometry)) return -1;
+    const mhaq_fq_iconv_geometry &g = *geometry;
+    const int64_t cp = (n_in + 15) / 16 * 16;
+    IgPlan l{};
+    int64_t bytes = (int64_t)g.kernel_h * g.kernel_w * cp;
+    if (!igroup_depthwise(n_in, n_out, g.groups)) {
+        l = igroup_plan(n_out, g.groups, n_in / g.groups, g.kernel_h, g.kernel_w);
+        bytes = (int64_t)l.n_tiles * l.k_stages * l.tile_n * kIcStageK;
+    }
+    if (n_tiles) *n_tiles = l.n_tiles;
+    if (tile_n) *tile_n = l.tile_n;
+    if (tile_out) *tile_out = l.tile_out;
+    if (groups_per_tile) *groups_per_tile = l.gpt;
+    if (tiles_per_group) *tiles_per_group = l.parts;
+    if (k_stages) *k_stages = l.k_stages;
+    return bytes;
+}
+
+int mhaq_fq_iconv_grouped_u8(const uint8_t *codes, const uint8_t *weights, const float *alpha, const float *beta,
+                             const float *ctab, const int32_t *h_class, const int32_t *w_class, int n_w_classes,
+                             int64_t batch, int64_t height, int64_t width, int64_t n_in, int64_t n_out,
+                             const mhaq_fq_iconv_geometry *geometry, int act_max_code, int weight_max_code,
+                             const mhaq_fq_iconv_epilogue *epilogue, void *stream) {
+    IConvArgs a;
+    IgPlan l;
+    int rc = igroup_args(codes, weights, alpha, beta, ctab, h_class, w_class, n_w_classes, batch, height, width,
+                         n_in, n_out, geometry, act_max_code, weight_max_code, epilogue, a, l);
+    if (rc) return rc;
+    if (igroup_depthwise(n_in, n_out, geometry->groups)) {
+        const int64_t blocks = (a.m * (a.cp / 16) + kDwThreads - 1) / kDwThreads;
+        const int grid = (int)(blocks < 148 * 64 ? blocks : 148 * 64);
+        fq_idw_kernel<<<grid, kDwThreads, 0, (cudaStream_t)stream>>>(a);
+        return last_error();
+    }
+    rc = iconv_smem_opt_in<true, true>();
+    if (rc) return rc;
+    const dim3 grid((unsigned)((a.m + kIcTileM - 1) / kIcTileM), (unsigned)l.n_tiles);
+    fq_iconv_kernel<true, true><<<grid, kIcThreads, iconv_smem_bytes(a.tile_n), (cudaStream_t)stream>>>(a);
     return last_error();
 }
 

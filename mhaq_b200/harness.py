@@ -225,11 +225,24 @@ def build_model(name: str, num_classes: Optional[int] = None) -> nn.Module:
         return CifarResNet(3, num_classes or 10)
     if name == "rfdn":
         return Rfdn(scale=4)
+    # grouped, depthwise and dilated networks (random weights; nothing is downloaded)
+    if name == "mobilenet_v2":
+        import torchvision
+        return torchvision.models.mobilenet_v2(num_classes=num_classes or 1000)
+    if name == "resnext50_32x4d":
+        import torchvision
+        return torchvision.models.resnext50_32x4d(num_classes=num_classes or 1000)
+    if name == "resnet50_dilated":      # the DeepLab backbone: layer3 / layer4 at dilation 2 / 4
+        import torchvision
+        return torchvision.models.resnet50(num_classes=num_classes or 1000,
+                                           replace_stride_with_dilation=[False, True, True])
     raise ValueError(name)
 
 
 EXCLUDED = {"resnet18": ("conv1", "fc"), "resnet20": ("conv1", "linear"),
-            "rfdn": ("fea_conv", "upsampler.0")}
+            "rfdn": ("fea_conv", "upsampler.0"),
+            "mobilenet_v2": ("features.0.0", "classifier.1"),
+            "resnext50_32x4d": ("conv1", "fc"), "resnet50_dilated": ("conv1", "fc")}
 
 
 # ------------------------------------------------------------------ calibration

@@ -1259,11 +1259,71 @@ def iconv_weight_operand(cw: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def tap_classes(size: int, k: int, stride: int, pad: int):
+def iconv_grouped_layout(n_in: int, n_out: int, kh: int, kw: int, groups: int):
+    """(bytes, n_tiles, tile_n, tile_out, groups_per_tile, tiles_per_group, k_stages) of the weight
+    operand of a grouped layer (mhaq_fq_iconv_grouped_weight_bytes); n_tiles = 0 for a depthwise one."""
+    g = _lib.IConvGeometry(kh, kw, 1, 1, 0, 0, 1, 1, groups)
+    ints = [ctypes.c_int() for _ in range(5)]
+    ks = ctypes.c_int64()
+    n = int(lib.mhaq_fq_iconv_grouped_weight_bytes(n_in, n_out, ctypes.byref(g), *(ctypes.byref(v) for v in ints),
+                                                   ctypes.byref(ks)))
+    if n < 0:
+        raise ValueError(f"iconv_grouped_layout: bad geometry n_in={n_in}, n_out={n_out}, groups={groups}")
+    return (n, *(v.value for v in ints), ks.value)
+
+
+def grouped_tile(t: int, groups: int, cin_g: int, cout_g: int, tile_out: int, gpt: int, parts: int):
+    """(n_base, n_here, first group, groups, first 16-channel chunk, chunks) of N tile ``t`` of a
+    grouped weight operand (the kernel's igroup_tile)."""
+    if parts == 1:
+        g_lo = t * gpt
+        g_hi = min(groups, g_lo + gpt)
+        n_base, n_end = g_lo * cout_g, g_hi * cout_g
+    else:
+        g_lo = t // parts
+        g_hi = g_lo + 1
+        n_base = g_lo * cout_g + (t % parts) * tile_out
+        n_end = min(n_base + tile_out, g_hi * cout_g)
+    c_lo = g_lo * cin_g // 16
+    return n_base, n_end - n_base, g_lo, g_hi - g_lo, c_lo, (g_hi * cin_g + 15) // 16 - c_lo
+
+
+def iconv_grouped_weight_operand(cw: torch.Tensor, groups: int) -> torch.Tensor:
+    """The weight operand of mhaq_fq_iconv_grouped_u8 from grouped weight codes
+    ``cw [N, C / groups, kh, kw]``: for a depthwise layer (groups == C == N) u8 ``[kh * kw][Cp]``,
+    otherwise block-diagonal N tiles (include/mhaq_fq.h), flat uint8."""
+    n, cin_g, kh, kw = cw.shape
+    cin, taps = cin_g * groups, kh * kw
+    cp = code_channels(cin)
+    nbytes, nt, tn, to, gpt, parts, ks = iconv_grouped_layout(cin, n, kh, kw, groups)
+    if nt == 0:
+        w = torch.zeros(taps, cp, dtype=torch.uint8, device=cw.device)
+        w[:, :cin] = cw[:, 0].reshape(n, taps).t().to(torch.uint8)
+        return w.reshape(-1)
+    cout_g = n // groups
+    cwt = cw.permute(0, 2, 3, 1).reshape(n, taps, cin_g).to(torch.uint8)
+    rows = torch.zeros(nt, tn, ks * 128, dtype=torch.uint8, device=cw.device)
+    for t in range(nt):
+        n_base, n_here, g_lo, n_grp, c_lo, kc = grouped_tile(t, groups, cin_g, cout_g, to, gpt, parts)
+        blk = torch.zeros(tn, taps, kc * 16, dtype=torch.uint8, device=cw.device)
+        for i in range(n_grp):
+            g = g_lo + i
+            lo = g * cin_g - c_lo * 16                       # the group's first K column of a tap
+            n0, n1 = max(n_base, g * cout_g), min(n_base + n_here, (g + 1) * cout_g)
+            blk[n0 - n_base:n1 - n_base, :, lo:lo + cin_g] = cwt[n0:n1]
+            blk[to + i, :, lo:lo + cin_g] = 1
+        rows[t, :, :taps * kc * 16] = blk.reshape(tn, -1)
+    out = rows.view(nt, tn // 8, 8, ks, 8, 16).permute(0, 3, 1, 4, 2, 5).reshape(-1)
+    assert out.numel() == nbytes
+    return out
+
+
+def tap_classes(size: int, k: int, stride: int, pad: int, dilation: int = 1):
     """Tap-validity classes along one axis: (class of each output position (int32 [out]),
-    valid taps of each class (bool [n_classes, k]))."""
-    out = (size + 2 * pad - k) // stride + 1
-    pos = torch.arange(out)[:, None] * stride - pad + torch.arange(k)[None, :]
+    valid taps of each class (bool [n_classes, k])).  Tap t of output o reads position
+    o * stride - pad + t * dilation."""
+    out = (size + 2 * pad - dilation * (k - 1) - 1) // stride + 1
+    pos = torch.arange(out)[:, None] * stride - pad + torch.arange(k)[None, :] * dilation
     valid = ((pos >= 0) & (pos < size)).to(torch.uint8)
     uniq, inv = torch.unique(valid, dim=0, return_inverse=True)
     return inv.to(torch.int32), uniq.bool()
@@ -1290,10 +1350,21 @@ class IntLayerOperands:
     bias: Optional[torch.Tensor]  # fp64 [N] or None
     tables: dict
     sa: float                     # activation scale
+    groups: int = 1               # weight: [N, cin / groups, kh, kw]
+    dilation: Tuple[int, int] = (1, 1)
 
     @property
     def cp(self) -> int:
         return code_channels(self.cin)
+
+    @property
+    def dense(self) -> bool:
+        """An ungrouped, undilated layer: mhaq_fq_iconv_u8 and its weight operand."""
+        return self.groups == 1 and tuple(self.dilation) == (1, 1)
+
+    def out_size(self, h: int, w: int, stride, padding) -> Tuple[int, int]:
+        return ((h + 2 * padding[0] - self.dilation[0] * (self.kh - 1) - 1) // stride[0] + 1,
+                (w + 2 * padding[1] - self.dilation[1] * (self.kw - 1) - 1) // stride[1] + 1)
 
     def fold_affine(self, k, shift) -> "IntLayerOperands":
         """Operands of ``k * y + shift`` (``k``, ``shift``: ``[N]``, taken in fp64), e.g. an eval
@@ -1311,11 +1382,12 @@ class IntLayerOperands:
                                    zpw=zpw, bias=bias, tables={})
 
     def constant_table(self, hvalid: torch.Tensor, wvalid: torch.Tensor) -> torch.Tensor:
-        """fp64 ctab [n_h_classes * n_w_classes][N]: zpa * (sw * sum_{k in p} cw + zpw * |p|) + bias."""
+        """fp64 ctab [n_h_classes * n_w_classes][N]: zpa * (sw * sum_{k in p} cw + zpw * |p|) + bias,
+        |p| = valid taps x input channels per group."""
         mask = (hvalid[:, None, :, None] & wvalid[None, :, None, :]).to(torch.float64)
         mask = mask.to(self.tap_sums.device)
         wsum = torch.einsum("hwab,nab->hwn", mask, self.tap_sums)
-        cnt = mask.sum((2, 3))[..., None] * self.cin
+        cnt = mask.sum((2, 3))[..., None] * (self.cin // self.groups)
         c = self.zpa * (self.sw * wsum + self.zpw * cnt)
         if self.bias is not None:
             c = c + self.bias
@@ -1326,8 +1398,8 @@ class IntLayerOperands:
         key = (h, w, tuple(stride), tuple(padding))
         t = self.tables.get(key)
         if t is None:
-            hc, hv = tap_classes(h, self.kh, stride[0], padding[0])
-            wc, wv = tap_classes(w, self.kw, stride[1], padding[1])
+            hc, hv = tap_classes(h, self.kh, stride[0], padding[0], self.dilation[0])
+            wc, wv = tap_classes(w, self.kw, stride[1], padding[1], self.dilation[1])
             dev = self.weight.device
             t = self.tables[key] = (hc.to(dev), wc.to(dev), wv.shape[0],
                                     self.constant_table(hv, wv).to(device=dev, dtype=torch.float32).contiguous())
@@ -1339,15 +1411,24 @@ def int32_bound_ok(k_bytes: int, a_top: int, w_top: int) -> bool:
     return k_bytes * a_top * w_top < (1 << 31)
 
 
-def int_layer_operands(cw, sw, zpw, sa, zpa, bias, a_top: int, w_top: int) -> IntLayerOperands:
-    """Operands of an integer layer on ``cw``'s device from the weight codes ``cw [N, C, kh, kw]``
-    (integers in [0, w_top]), the weight scale / zero point (``[N]`` or one element), the
+def int_layer_operands(cw, sw, zpw, sa, zpa, bias, a_top: int, w_top: int, groups: int = 1,
+                       dilation=1) -> IntLayerOperands:
+    """Operands of an integer layer on ``cw``'s device from the weight codes ``cw [N, C / groups, kh,
+    kw]`` (integers in [0, w_top]), the weight scale / zero point (``[N]`` or one element), the
     activation scale / zero point (floats) and the layer's bias (``[N]`` or None).  alpha and beta
-    are formed in fp64 and rounded once to fp32."""
-    n, c, kh, kw = cw.shape
+    are formed in fp64 and rounded once to fp32.  A grouped or dilated layer gets the weight operand
+    of mhaq_fq_iconv_grouped_u8 (``iconv_grouped_weight_operand``)."""
+    n, c_g, kh, kw = cw.shape
+    dilation = _pair(dilation)
+    c = c_g * groups
+    if groups < 1 or n % groups or min(dilation) < 1:
+        raise ValueError(f"integer layer: groups={groups} must divide the {n} output channels and the "
+                         f"dilation {dilation} be at least 1")
     if not (1 <= a_top <= 255 and 1 <= w_top <= 255):
         raise ValueError(f"integer layer: code bounds must lie in [1, 255], got {a_top} and {w_top}")
-    if not int32_bound_ok(kh * kw * code_channels(c), a_top, w_top):
+    dense = groups == 1 and dilation == (1, 1)
+    # a grouped / dilated channel sums kh * kw * C / groups products (no padding channels)
+    if not int32_bound_ok(kh * kw * (code_channels(c) if dense else c_g), a_top, w_top):
         raise ValueError("integer layer: K * (n_levels - 1) * (2^bits - 1) >= 2^31 would overflow the "
                          "int32 accumulator")
     dev = cw.device
@@ -1356,11 +1437,12 @@ def int_layer_operands(cw, sw, zpw, sa, zpa, bias, a_top: int, w_top: int) -> In
     zpw = torch.as_tensor(zpw).to(**f64).reshape(-1).expand(n).contiguous()
     sa, zpa = float(sa), float(zpa)
     return IntLayerOperands(
-        weight=iconv_weight_operand(cw), alpha=(sa * sw).float(), beta=(sa * zpw).float(),
+        weight=iconv_weight_operand(cw) if dense else iconv_grouped_weight_operand(cw, groups),
+        alpha=(sa * sw).float(), beta=(sa * zpw).float(),
         n_out=n, cin=c, kh=kh, kw=kw, a_top=a_top, w_top=w_top,
         tap_sums=cw.to(**f64).sum(1), sw=sw, zpw=zpw, zpa=zpa,
         bias=None if bias is None else torch.as_tensor(bias).to(**f64).reshape(n),
-        tables={}, sa=sa)
+        tables={}, sa=sa, groups=groups, dilation=dilation)
 
 
 def batchnorm_foldable(bn) -> bool:
@@ -1403,9 +1485,21 @@ def _pair(v):
     return (int(v), int(v)) if isinstance(v, int) else (int(v[0]), int(v[1]))
 
 
-def int_conv2d(codes, L: IntLayerOperands, stride=1, padding=0) -> torch.Tensor:
+def _check_geometry(L: IntLayerOperands, dilation, groups):
+    if dilation is not None and _pair(dilation) != tuple(L.dilation):
+        raise ValueError(f"integer layer: dilation {_pair(dilation)} differs from the operands' {tuple(L.dilation)}")
+    if groups is not None and int(groups) != L.groups:
+        raise ValueError(f"integer layer: groups={groups} differs from the operands' {L.groups}")
+
+
+def int_conv2d(codes, L: IntLayerOperands, stride=1, padding=0, dilation=None, groups=None) -> torch.Tensor:
     """fp32 convolution of activation codes ``[B, H, W, Cp]`` (``act_codes``) with the layer's
-    operands: a channels_last ``[B, N, Ho, Wo]`` tensor."""
+    operands: a channels_last ``[B, N, Ho, Wo]`` tensor.  ``dilation`` and ``groups`` are those of
+    ``L`` (None: as given there; another value raises).  A grouped or dilated layer runs
+    mhaq_fq_iconv_grouped_u8 (depthwise on the CUDA cores, the rest on the tensor cores)."""
+    _check_geometry(L, dilation, groups)
+    if not L.dense:
+        return int_conv2d_fused(codes, L, stride, padding)[0]
     b, h, w, _ = codes.shape
     stride, padding = _pair(stride), _pair(padding)
     ho = (h + 2 * padding[0] - L.kh) // stride[0] + 1
@@ -1418,23 +1512,24 @@ def int_conv2d(codes, L: IntLayerOperands, stride=1, padding=0) -> torch.Tensor:
 ACTIVATIONS = {None: _lib.ACT_NONE, "relu": _lib.ACT_RELU, "leaky_relu": _lib.ACT_LEAKY_RELU}
 
 
-def int_conv2d_fused(codes, L: IntLayerOperands, stride=1, padding=0, *, residual=None, activation=None,
-                     negative_slope=None, out_fp32=True, code_params=None):
+def int_conv2d_fused(codes, L: IntLayerOperands, stride=1, padding=0, dilation=None, groups=None, *,
+                     residual=None, activation=None, negative_slope=None, out_fp32=True, code_params=None):
     """``int_conv2d`` with its epilogue extended (mhaq_fq_iconv_fused_u8): t = the convolution
     (with whatever ``fold_batchnorm`` folded into ``L``), then ``t + residual`` (fp32, the output's
     shape; made channels_last-contiguous, which copies an NCHW tensor), then ``activation``
     (None, "relu" or "leaky_relu" with ``negative_slope``, default 0.01), one launch.  Returns
     ``(y, codes)``: y the channels_last fp32 ``[B, N, Ho, Wo]`` if ``out_fp32``, codes the uint8
     ``[B, Ho, Wo, code_channels(N)]`` of the next ``NoisyAct`` if ``code_params`` = (scale,
-    zero_point, max_val) is given (as ``act_codes`` would make them from y), else None."""
+    zero_point, max_val) is given (as ``act_codes`` would make them from y), else None.
+    ``dilation`` and ``groups`` as in ``int_conv2d``."""
+    _check_geometry(L, dilation, groups)
     if activation not in ACTIVATIONS:
         raise ValueError(f"int_conv2d_fused: unknown activation {activation!r}")
     if not out_fp32 and code_params is None:
         raise ValueError("int_conv2d_fused: no output requested")
     b, h, w, _ = codes.shape
     stride, padding = _pair(stride), _pair(padding)
-    ho = (h + 2 * padding[0] - L.kh) // stride[0] + 1
-    wo = (w + 2 * padding[1] - L.kw) // stride[1] + 1
+    ho, wo = L.out_size(h, w, stride, padding)
     dev = codes.device
     y = torch.empty((b, L.n_out, ho, wo), dtype=torch.float32, device=dev,
                     memory_format=torch.channels_last) if out_fp32 else None
@@ -1459,6 +1554,14 @@ def int_conv2d_fused(codes, L: IntLayerOperands, stride=1, padding=0, *, residua
         slope = 0.01 if negative_slope is None else float(negative_slope)
         epi = _lib.IConvEpilogue(_ptr(residual), ACTIVATIONS[activation], slope, _ptr(y), _ptr(out_codes),
                                  *(_ptr(p) for p in prm))
+        if not L.dense:
+            geo = _lib.IConvGeometry(L.kh, L.kw, stride[0], stride[1], padding[0], padding[1], L.dilation[0],
+                                     L.dilation[1], L.groups)
+            _check_rc(lib.mhaq_fq_iconv_grouped_u8(_ptr(codes), _ptr(L.weight), _ptr(L.alpha), _ptr(L.beta),
+                                                   _ptr(ctab), _ptr(hc), _ptr(wc), nwc, b, h, w, L.cin, L.n_out,
+                                                   ctypes.byref(geo), L.a_top, L.w_top, ctypes.byref(epi),
+                                                   _stream()), "mhaq_fq_iconv_grouped_u8")
+            return y, out_codes
         _check_rc(lib.mhaq_fq_iconv_fused_u8(_ptr(codes), _ptr(L.weight), _ptr(L.alpha), _ptr(L.beta), _ptr(ctab),
                                              _ptr(hc), _ptr(wc), nwc, b, h, w, L.cp, L.n_out, L.kh, L.kw,
                                              stride[0], stride[1], padding[0], padding[1], L.a_top, L.w_top,

@@ -8,7 +8,8 @@ to uint8 activation codes and runs an int8 tensor-core GEMM against the exported
 (include/mhaq_fq.h "Integer layers", DESIGN §3).  Everything between those layers (BN, ReLU,
 pooling, residual adds, unquantized layers) stays as it is.
 
-The convolution geometry (stride, padding) comes from the model's modules; every number comes
+The convolution geometry (stride, padding, and with ``allow_groups_and_dilation=True`` groups and
+dilation) comes from the model's modules; every number comes
 from the blob: the weight codes are unpacked from the packed format with integer operations, never
 re-derived from dequantized floats.
 """
@@ -64,6 +65,7 @@ class IntegerConv2d(_IntegerLayer):
     def __init__(self, act, operands, stride, padding):
         super().__init__(act, operands)
         self.stride, self.padding = tuple(stride), tuple(padding)
+        self.dilation, self.groups = tuple(operands.dilation), operands.groups
 
     def forward(self, x):
         codes, _ = ops.act_codes(x, self.act_scale, self.act_zero_point, self.act_max_val)
@@ -85,8 +87,9 @@ def _qscheme(m):
     return "PER_CHANNEL" if is_per_channel(m.qscheme) else "PER_TENSOR"
 
 
-def _check_pair(name, act_e, w, we):
-    """ValueError naming the layer for everything the integer kernels cannot run exactly."""
+def _check_pair(name, act_e, w, we, allow_groups_and_dilation=False):
+    """ValueError naming the layer for everything the integer kernels cannot run exactly (grouped
+    and dilated convolutions unless ``allow_groups_and_dilation``)."""
     if act_e["disabled"]:
         raise ValueError(f"build_integer_model: {name}: the activation quantizer is disabled (act_bit = -1); "
                          "an integer layer needs activation codes")
@@ -97,27 +100,31 @@ def _check_pair(name, act_e, w, we):
     if list(w.weight.shape) != list(we["shape"]) or we["qscheme"] != _qscheme(w):
         raise ValueError(f"build_integer_model: {name}: the model's layer differs from the export's "
                          "(shape or qscheme)")
+    dense = not isinstance(w, NoisyConv2d) or (w.groups == 1 and tuple(w.dilation) == (1, 1))
     if isinstance(w, NoisyConv2d):
-        if w.groups != 1 or tuple(w.dilation) != (1, 1):
+        if not dense and not allow_groups_and_dilation:
             raise ValueError(f"build_integer_model: {name}: grouped or dilated convolutions are not supported")
         if w.padding_mode != "zeros" or isinstance(w.padding, str):
             raise ValueError(f"build_integer_model: {name}: only explicit zero padding is supported "
                              f"(padding_mode={w.padding_mode!r}, padding={w.padding!r})")
     kk = w.weight[0, 0].numel() if w.weight.dim() == 4 else 1
-    k_bytes = kk * ops.code_channels(w.weight.shape[1])
+    # a grouped / dilated channel sums kh * kw * (C / groups) products, without padding channels
+    k_bytes = kk * (ops.code_channels(w.weight.shape[1]) if dense else w.weight.shape[1])
     if not ops.int32_bound_ok(k_bytes, max(1, act_e["n_levels"] - 1), (1 << we["bits"]) - 1):
         raise ValueError(f"build_integer_model: {name}: K * (n_levels - 1) * (2^bits - 1) >= 2^31 would "
                          "overflow the int32 accumulator")
 
 
-def _integer_layer(name, act_e, w, we):
-    _check_pair(name, act_e, w, we)
+def _integer_layer(name, act_e, w, we, allow_groups_and_dilation=False):
+    _check_pair(name, act_e, w, we, allow_groups_and_dilation)
     dev = w.weight.device
     cw = unpack_weight_codes(we).to(dev)
     if cw.dim() == 2:
         cw = cw[:, :, None, None]
+    geo = dict(groups=w.groups, dilation=tuple(w.dilation)) if isinstance(w, NoisyConv2d) else {}
     ops_ = ops.int_layer_operands(cw, we["scale"], we["zero_point"], act_e["scale"], act_e["zero_point"],
-                                  we["bias"], a_top=max(1, act_e["n_levels"] - 1), w_top=(1 << we["bits"]) - 1)
+                                  we["bias"], a_top=max(1, act_e["n_levels"] - 1), w_top=(1 << we["bits"]) - 1,
+                                  **geo)
     if isinstance(w, NoisyConv2d):
         return IntegerConv2d(act_e, ops_, w.stride, w.padding)
     return IntegerLinear(act_e, ops_)
@@ -136,10 +143,14 @@ def _tree_copy(m: nn.Module) -> nn.Module:
 
 
 @torch.no_grad()
-def build_integer_model(model, blob) -> nn.Module:
+def build_integer_model(model, blob, *, allow_groups_and_dilation=False) -> nn.Module:
     """An eval-mode copy of ``model`` whose quantized layers run on the integer codes of ``blob``
     (from ``export_quantized``); the other layers share their parameters with ``model``.  ``model`` must have the exporter's architecture; every mismatch
-    and every layer the integer kernels cannot run raises ValueError naming the layer."""
+    and every layer the integer kernels cannot run raises ValueError naming the layer.
+
+    Grouped and dilated convolutions are refused unless ``allow_groups_and_dilation=True``; with it
+    they become integer layers too (``ops.int_conv2d``: depthwise layers on the CUDA cores, the
+    other grouped and dilated layers on the tensor cores)."""
     if blob.get("format") != FORMAT or blob.get("version") != VERSION:
         raise ValueError(f"build_integer_model: not a {FORMAT} v{VERSION} export")
     mods = {n: m for n, m in model.named_modules() if _layer_kind(m) is not None}
@@ -156,7 +167,7 @@ def build_integer_model(model, blob) -> nn.Module:
                 and isinstance(getattr(m, "0"), (NoisyConv2d, NoisyLinear)):
             pre = f"{n}." if n else ""
             pairs.append((n, layers[pre + "activations_quantizer"], getattr(m, "0"), layers[pre + "0"]))
-    built = {n: _integer_layer(n, ae, w, we) for n, ae, w, we in pairs}     # validates all before copying
+    built = {n: _integer_layer(n, ae, w, we, allow_groups_and_dilation) for n, ae, w, we in pairs}     # validates all before copying
     out = _tree_copy(model).eval()
     for n, layer in built.items():
         parent, _, leaf = n.rpartition(".")
@@ -202,7 +213,7 @@ def _as_add_operand(r, codes, L, stride, padding):
     is exact for every such dtype, and torch converts the same way before it adds).  Anything
     else is left to ``int_conv2d_fused`` to refuse."""
     b, h, w, _ = codes.shape
-    out = (b, L.n_out, (h + 2 * padding[0] - L.kh) // stride[0] + 1, (w + 2 * padding[1] - L.kw) // stride[1] + 1)
+    out = (b, L.n_out, *L.out_size(h, w, stride, padding))
     if (not isinstance(r, torch.Tensor) or torch.promote_types(r.dtype, torch.float32) != torch.float32
             or (r.dtype == torch.float32 and tuple(r.shape) == out)):
         return r
